@@ -5,6 +5,7 @@ alpha compositing, forward + backward) on B200, through the reference-facing dro
     python bench.py --gpus 1 --steps 20 --warmup 5            # our arm (one JSON line)
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1   # the reference's algorithm on host cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # weak scaling, rays sharded
+    python bench.py --steps 20 --warmup 5 --dump-outputs DIR   # + the last timed step's outputs as DIR/*.npy
 
 A "step" = Volume_Renderer.vol_render(...) + MSE(Cr)+MSE(Cf) + loss.backward() on one batch of synthetic rays
 (BASELINE.json configs[1]: 4096 rays x 128 samples, L=16 F=2 T=2^19, lego-shaped 800x800 scene).  The optimiser
@@ -217,8 +218,8 @@ def measured_peaks():
 
 
 # ---------------------------------------------------------------------------------------------------------------
-# CPU arm: the reference ITSELF (unmodified modules from baseline/_ref or /root/reference, loaded by oracle/ref_loader.py
-# with environment shims only) on the box's host cores; oracle/port.py only when no reference tree can be found.
+# CPU arm: the reference ITSELF (unmodified modules from the copy build() staged in oracle/_ref, loaded by
+# oracle/ref_loader.py with environment shims only) on the box's host cores; oracle/port.py only when there is no copy.
 # ---------------------------------------------------------------------------------------------------------------
 def _reference_modules():
     from oracle import ref_loader
@@ -338,6 +339,31 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_ROWS = 1 << 17
+
+
+def _dump_sample(x, dim):
+    """x cut to a fixed seeded sample of DUMP_ROWS indices (ascending) along dim; whole when it has no more."""
+    n = x.shape[dim]
+    if n <= DUMP_ROWS:
+        return x
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    return x.index_select(dim, idx.to(x.device))
+
+
+def dump_outputs(path, outputs, enc, mlp):
+    """--dump-outputs: what the last timed step hands its caller -- the loss, the colours of both passes and the parameter
+    gradients -- as float32 DIR/<name>.npy.  Colours keep a fixed seeded sample of DUMP_ROWS rays and the table gradient
+    (L, T, F) one of DUMP_ROWS table rows (the same rows on every level), so that the files stay far below 64 MB."""
+    arrays = {"loss": outputs["loss"].reshape(1), "rgb_coarse": _dump_sample(outputs["rgb_coarse"], 0),
+              "rgb_fine": _dump_sample(outputs["rgb_fine"], 0),
+              "grad.hash_tables": _dump_sample(torch.stack([e.weight.grad for e in enc.Embedding_list]), 1)}
+    arrays.update({f"grad.{n}": p.grad for n, p in mlp.named_parameters()})
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.detach().float().cpu().numpy())
+
+
 # ---------------------------------------------------------------------------------------------------------------
 def run_b200(args):
     import human_body_reconstruction_b200 as hbr
@@ -399,6 +425,11 @@ def run_b200(args):
     if args.precision == "f16":
         mlp.tc_grad_scale = 65536.0                # fp16 operands: what GradScaler's initial scale does in train_hash2.py:192,226
 
+    outputs = {}                                   # --dump-outputs: colours and loss of the last step (detached)
+
+    def keep(Cr, Cf, loss):
+        outputs.update(rgb_coarse=Cr.detach(), rgb_fine=Cf.detach(), loss=loss.detach())
+
     def step(batch):
         o, d, n, gt = batch
         for p in params:
@@ -408,6 +439,16 @@ def run_b200(args):
                                       hierarchical=args.hierarchical)
             loss = default_loss(Cr, Cf, gt)                       # MSE(Cr) + MSE(Cf), train_hash2.py:221 (one fused kernel)
         loss.backward()
+        if args.dump_outputs:
+            keep(Cr, Cf, loss)
+        return loss
+
+    def graph_loss(Cr, Cf, gt):
+        """default_loss; during the capture it also keeps the tensors that every replay writes colours and loss into (the
+        eager warm-up passes of GraphedStep.capture() keep nothing)."""
+        loss = default_loss(Cr, Cf, gt)
+        if args.dump_outputs and torch.cuda.is_current_stream_capturing():
+            keep(Cr, Cf, loss)
         return loss
 
     def barrier():
@@ -450,7 +491,9 @@ def run_b200(args):
     if args.graph in ("on", "auto"):
         try:
             from human_body_reconstruction_b200.graph import GraphedStep
-            gs = GraphedStep(vr, nerf, params, rays, args.samples, args.hierarchical, dev, autocast=amp, autocast_dtype=amp_dtype).capture()
+            outputs.clear()                                                # nothing of an eager step is released mid-capture
+            gs = GraphedStep(vr, nerf, params, rays, args.samples, args.hierarchical, dev, loss_fn=graph_loss, autocast=amp,
+                             autocast_dtype=amp_dtype).capture()
             host_packed = [GraphedStep.pack_batch(*b, pin=True) for b in host]       # one H2D copy per step
             resident_packed = [p.to(dev) for p in host_packed]
             for k in range(3):
@@ -466,6 +509,8 @@ def run_b200(args):
     run = (lambda k: gs(resident_packed[k % len(resident_packed)])) if gs is not None else (lambda k: step(resident[k % len(resident)]))
     region_ms = sorted(timed_region(run) for _ in range(max(1, args.repeats)))
     dev_ms = region_ms[len(region_ms) // 2]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs, enc, mlp)      # before the steps below overwrite the gradients
 
     # (3) end to end: pinned host batch -> H2D -> step -> loss.item()
     e2e_s = 0.0
@@ -997,7 +1042,11 @@ def main():
     ap.add_argument("--no-c3", dest="c3", action="store_false", help="skip the configs[2] leg (2^20 rays/step global; 2^17 at N=1)")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="replay the step from a CUDA graph (auto = on; falls back to eager if capture fails)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (loss, "
+                    "colours, parameter gradients; seeded samples of the large ones) as float32 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE ONLY.  Generates tests/golden/*.npz by executing the UNMODIFIED reference
-(/root/reference, CPU, through oracle/ref_loader.py).  Run in the build container:
+(CPU, through oracle/ref_loader.py: the copy build() staged in oracle/_ref, or the checkout HBR_REFERENCE_DIR names):
 
     python oracle/make_golden.py
 

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY: CPU restatement ("port") of the reference NeRF hot path.
 
 Nothing in the product package may import this module.  It exists so that the CUDA path
-can be checked on a machine where /root/reference does not exist (the GPU box).  Allowed
+can be checked without a checkout of the reference.  Allowed
 importers: tests/, __graft_entry__.smoke(), and bench.py's cpu_baseline / --impl reference legs.
 
 Parity status: PINNED.  The reference ships no tests or golden vectors (SURVEY.md section 4),

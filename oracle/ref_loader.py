@@ -1,9 +1,10 @@
 """TEST INFRASTRUCTURE ONLY -- never imported by the product package.
 
-Loads the *unmodified* reference modules from /root/reference on the CPU so that
+Loads the *unmodified* reference modules on the CPU -- from the checkout HBR_REFERENCE_DIR names, else from the
+verbatim copy __graft_entry__.build() stages in oracle/_ref (git-ignored) -- so that
 (a) `oracle/make_golden.py` can generate the committed fixtures in tests/golden/ and
-(b) the CPU test-suite can pin `oracle/port.py` against the live reference when the
-    reference tree happens to be present (it is NOT present on the GPU box).
+(b) bench.py's reference arm and the drop-in script tests run the reference itself (without a copy they use
+    oracle/port.py or skip).
 
 The shims are environmental only (SURVEY.md appendix B); no reference arithmetic is touched:
   * h5py / matplotlib are imported-but-unused by vol_renderer.py:4,6 and helper.py:7-8 -> empty stubs
@@ -19,20 +20,8 @@ import types
 
 import numpy as np
 
-_ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _find_reference() -> str:
-    """HBR_REFERENCE_DIR, else the read-only checkout of the build container, else the verbatim copy that
-    __graft_entry__.build() stages under baseline/_ref (git-ignored; the only one that exists on the GPU box)."""
-    cands = [os.environ.get("HBR_REFERENCE_DIR"), "/root/reference", os.path.join(_ROOT, "baseline", "_ref")]
-    for c in cands:
-        if c and os.path.isfile(os.path.join(c, "hash_encoding.py")):
-            return c
-    return cands[1]
-
-
-REF_DIR = _find_reference()
+STAGED_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+REF_DIR = os.environ.get("HBR_REFERENCE_DIR") or STAGED_DIR
 
 
 def available() -> bool:

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, load_golden
+from conftest import GOLDEN, load_golden, mlp_params
 from human_body_reconstruction_b200 import formats
 
 
@@ -86,8 +86,26 @@ def test_checkpoint_names_and_dataparallel_prefix(tmp_path):
     assert list(torch.load(n_path).keys())[0] == "module.sig_model.0.weight"      # the reference's key (train_hash2.py:127,299)
     bare, enc2 = Net(), torch.nn.Embedding(4, 2)
     formats.load_checkpoint(name, bare, enc2)                                     # prefix stripped for an unwrapped module
-    assert torch.equal(bare.sig_model[0].weight, net.module.sig_model[0].weight) and torch.equal(enc2.weight, enc.weight)
+    # nn.DataParallel moves its module to cuda:0 where there is a GPU: the weights are compared on the host
+    assert torch.equal(bare.sig_model[0].weight, net.module.sig_model[0].weight.cpu()) and torch.equal(enc2.weight, enc.weight)
     torch.save(bare.state_dict(), n_path)
     wrapped = torch.nn.DataParallel(Net())
     formats.load_checkpoint(name, wrapped, enc2)                                  # and added for a wrapped one
-    assert torch.equal(wrapped.module.sig_model[0].weight, bare.sig_model[0].weight)
+    assert torch.equal(wrapped.module.sig_model[0].weight.cpu(), bare.sig_model[0].weight)
+
+
+def test_checkpoint_keys_and_shapes_match_the_reference_classes(tmp_path):
+    """What train_hash2.py:299-300 saves from the drop-in classes has the keys and shapes of the reference's own: its
+    MLP_3D state_dict (tests/golden/mlp.npz, written by the unmodified reference) behind nn.DataParallel's prefix, and one
+    (T, F) table per level of its HashEncoder.Embedding_list (tests/golden/hash_pow2.npz: L=16, T=1024, F=2)."""
+    import human_body_reconstruction_b200 as hbr
+    L, T, F = load_golden("hash_pow2.npz")["tables"].shape
+    enc = hbr.HashEncoder(N_min=16, N_max=2048.0, L=L, F=F, T=T, dim=3, mu=torch.zeros(3), sigma=torch.tensor(1.0))
+    mlp = hbr.MLP_3D(num_sig=2, num_col=2, L=L, F=F, d_view=24, max_bound=torch.ones(3), min_bound=-torch.ones(3))
+    name = str(tmp_path / "m")
+    formats.save_checkpoint(name, torch.nn.DataParallel(mlp), enc)
+    n_path, e_path = formats.checkpoint_paths(name)
+    nerf, encd = torch.load(n_path, map_location="cpu"), torch.load(e_path, map_location="cpu")
+    ref_mlp = mlp_params(load_golden("mlp.npz"))
+    assert {k: tuple(v.shape) for k, v in nerf.items()} == {"module." + k: tuple(v.shape) for k, v in ref_mlp.items()}
+    assert {k: tuple(v.shape) for k, v in encd.items()} == {f"Embedding_list.{i}.weight": (T, F) for i in range(L)}

@@ -1,8 +1,9 @@
 """GPU tests (-m gpu): the reference's UNMODIFIED scripts run on the drop-in modules through launch.py.
 
-train_hash2.py (the live trainer) and nerf2mesh.py are executed from baseline/_ref -- a verbatim copy of the reference
-checkout staged by __graft_entry__.build(); skipped when it is absent -- with launch.py building the import path
-(dropin/ in front of the script directory).  Checked: the hot-path modules really came from dropin/, the sm_100a kernels
+train_hash2.py (the live trainer) and nerf2mesh.py are executed from oracle/_ref -- the verbatim copy of the reference
+checkout that __graft_entry__.build() stages (or the checkout HBR_REFERENCE_DIR names); the scripts are not part of this
+repository, so the tests skip where no copy was staged -- with launch.py building the import path (dropin/ in front of
+the script directory).  Checked: the hot-path modules really came from dropin/, the sm_100a kernels
 really ran (C-ABI call counters), and the files the scripts write (bounds_model.npy, *_Nerf_hash.pth, *_encoder_hash.pth,
 density_grid_w_rgb.npy, the mesh) have the reference's names, keys and shapes.
 """
@@ -16,13 +17,14 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, ROOT
-from oracle import port
+from conftest import GOLDEN, ROOT, load_golden, mlp_params
+from oracle import port, ref_loader
 
 pytestmark = pytest.mark.gpu
-REF = os.path.join(ROOT, "baseline", "_ref")
-needs_ref = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "train_hash2.py")),
-                               reason="baseline/_ref (copy of the reference staged by __graft_entry__.build()) is absent")
+REF = ref_loader.REF_DIR
+HAVE_REF = os.path.isfile(os.path.join(REF, "train_hash2.py"))
+needs_ref = pytest.mark.skipif(not HAVE_REF, reason=f"runs the reference's own scripts: no reference copy at {REF} "
+                               "(build() stages one where a reference checkout is present)")
 
 RUNNER = r"""
 import json, os, sys
@@ -54,8 +56,8 @@ def trained(tmp_path_factory):
     """~20 steps of the unmodified train_hash2.py on the 2-view 5x6 scene (tests/golden/scene_new, the captured-humans
     json flavour), fp16 autocast + GradScaler as the script does, with --write so that it renders a test view and saves
     the checkpoints on its first iteration."""
-    if not os.path.isfile(os.path.join(REF, "train_hash2.py")):
-        pytest.skip("baseline/_ref absent")
+    if not HAVE_REF:
+        pytest.skip(f"no reference copy at {REF}")
     work = tmp_path_factory.mktemp("train")
     scene = os.path.join(work, "scene")
     shutil.copytree(os.path.join(GOLDEN, "scene_new"), scene)
@@ -94,11 +96,12 @@ def test_train_hash2_runs_unmodified_on_the_dropins(trained):
     encd = torch.load(os.path.join(work, "m_encoder_hash.pth"), map_location="cpu")
     want = [f"module.{n}.{i}.{w}" for n in ("sig_model", "col_model") for i in (0, 2, 4) for w in ("weight", "bias")]
     assert sorted(nerf.keys()) == sorted(want)
+    # keys and shapes of the reference MLP_3D's own state_dict (tests/golden/mlp.npz, written by the unmodified reference)
+    assert {k: tuple(v.shape) for k, v in nerf.items()} == {"module." + k: tuple(v.shape) for k, v in mlp_params(load_golden("mlp.npz")).items()}
     assert sorted(encd.keys()) == sorted(f"Embedding_list.{i}.weight" for i in range(16))
     assert all(tuple(v.shape) == (2 ** 12, 2) and v.dtype == torch.float32 for v in encd.values())
     assert all(torch.isfinite(v).all() for v in list(nerf.values()) + list(encd.values()))
-    # the checkpoint loads into the REFERENCE's own classes (same keys / shapes)
-    from oracle import ref_loader
+    # the checkpoint loads into the REFERENCE's own classes (same keys / shapes), from the same staged copy as the script
     if ref_loader.available():
         ref = ref_loader.load()
         with ref_loader.quiet():
