@@ -92,11 +92,15 @@ __device__ __forceinline__ SampleIn load_sample(const float* __restrict__ tr, co
   return q;
 }
 
+// MAPS: also depth = sum_s w_s t_s and opacity = sum_s w_s per ray (either pointer may be NULL); without it the kernel is
+// exactly the colour-only compositor (hbr_composite_fwd), the maps code is compiled out.
+template <bool MAPS>
 __global__ void __launch_bounds__(kRaysPerCta * 32)
 composite_fwd_kernel(const float* __restrict__ t, long long t_rs, const float* __restrict__ rgb, long long rgb_st,
                      const float* __restrict__ sigma, long long sig_st, const float* __restrict__ dn, float dn_scalar,
                      const uint8_t* __restrict__ mask, const int32_t* __restrict__ rowmap, long long R, int S,
-                     float* __restrict__ C, float* __restrict__ w_out, float ert_tau) {
+                     float* __restrict__ C, float* __restrict__ w_out, float ert_tau, float* __restrict__ depth,
+                     float* __restrict__ opac) {
   // ert_tau: early ray termination (opt-in; +inf = off, the reference's behaviour).  Once the optical depth accumulated
   // over whole 32-sample chunks exceeds ert_tau the remaining chunks are skipped and get weight 0.  With the default
   // threshold 104 the transmittance exp(-depth) of every skipped sample is EXACTLY 0 in fp32 (exp(-104) underflows), so
@@ -107,7 +111,7 @@ composite_fwd_kernel(const float* __restrict__ t, long long t_rs, const float* _
   if (ray >= R) return;
   const float* tr = t + ray * t_rs;
   const float dnr = dn ? __ldg(dn + ray) : dn_scalar;
-  float carry = 0.f, c0 = 0.f, c1 = 0.f, c2 = 0.f;
+  float carry = 0.f, c0 = 0.f, c1 = 0.f, c2 = 0.f, dsum = 0.f, asum = 0.f;
   for (int s0 = 0; s0 < S; s0 += 32) {
     const int s = s0 + lane;
     const long long gs = ray * S + s;
@@ -122,6 +126,10 @@ composite_fwd_kernel(const float* __restrict__ t, long long t_rs, const float* _
     const float w = s < S ? __fmul_rn(T, alpha) : 0.f;                   // :102
     if (s < S) {
       if (w_out) w_out[gs] = w;
+      if (MAPS) {
+        dsum += w * __ldg(tr + s);
+        asum += w;
+      }
       if (live) {
         const float* c = rgb + row * rgb_st;
         c0 += w * __ldg(c + 0);
@@ -138,22 +146,37 @@ composite_fwd_kernel(const float* __restrict__ t, long long t_rs, const float* _
   }
   c0 = warp_sum(c0); c1 = warp_sum(c1); c2 = warp_sum(c2);
   if (lane == 0) { C[ray * 3 + 0] = c0; C[ray * 3 + 1] = c1; C[ray * 3 + 2] = c2; }
+  if (MAPS) {
+    dsum = warp_sum(dsum); asum = warp_sum(asum);
+    if (lane == 0) {
+      if (depth) depth[ray] = dsum;
+      if (opac) opac[ray] = asum;
+    }
+  }
 }
 
 // ---- calc_color backward (SURVEY A.3) -------------------------------------------------------------------
-template <int NCH>
+// MAPS: per-ray gradients gD of depth = sum w t and gA of opacity = sum w enter the per-sample term as
+// c_s = g.rgb_s + gD t_s + gA (NULL = 0; gC may be NULL too); d(rgb) = w g is unchanged.  Without MAPS the code is compiled
+// out and the kernel is exactly hbr_composite_bwd's.
+template <int NCH, bool MAPS>
 __global__ void __launch_bounds__(kRaysPerCta * 32)
 composite_bwd_kernel(const float* __restrict__ t, long long t_rs, const float* __restrict__ rgb, long long rgb_st,
                      const float* __restrict__ sigma, long long sig_st, const float* __restrict__ dn, float dn_scalar,
                      const uint8_t* __restrict__ mask, const int32_t* __restrict__ rowmap, long long R, int S,
                      const float* __restrict__ gC, float* __restrict__ drgb, long long drgb_st, float* __restrict__ dsig,
-                     long long dsig_st, float ert_tau) {
+                     long long dsig_st, float ert_tau, const float* __restrict__ gD, const float* __restrict__ gA) {
   const int lane = threadIdx.x & 31;
   const long long ray = (long long)blockIdx.x * kRaysPerCta + (threadIdx.x >> 5);
   if (ray >= R) return;
   const float* tr = t + ray * t_rs;
   const float dnr = dn ? __ldg(dn + ray) : dn_scalar;
-  const float g0 = __ldg(gC + ray * 3 + 0), g1 = __ldg(gC + ray * 3 + 1), g2 = __ldg(gC + ray * 3 + 2);
+  float g0 = 0.f, g1 = 0.f, g2 = 0.f, gd = 0.f, ga = 0.f;
+  if (!MAPS || gC) { g0 = __ldg(gC + ray * 3 + 0); g1 = __ldg(gC + ray * 3 + 1); g2 = __ldg(gC + ray * 3 + 2); }
+  if (MAPS) {
+    if (gD) gd = __ldg(gD + ray);
+    if (gA) ga = __ldg(gA + ray);
+  }
   const bool packed = drgb_st == 4 && dsig_st == 4 && dsig == drgb + 3;
 
   float Tk[NCH], ek[NCH], ck[NCH], dk[NCH];     // transmittance, exp(-p), g.rgb, delta*[keep]
@@ -180,6 +203,7 @@ composite_bwd_kernel(const float* __restrict__ t, long long t_rs, const float* _
           ck[i] = g0 * __ldg(c + 0) + g1 * __ldg(c + 1) + g2 * __ldg(c + 2);
           dk[i] = q.keep ? q.delta : 0.f;
         }
+        if (MAPS) ck[i] = __fadd_rn(__fmaf_rn(gd, __ldg(tr + s), ck[i]), ga);   // gD = gA = 0: ck unchanged
       }
       done = carry > ert_tau;                    // warp-uniform; skipped chunks keep T = 0: zero weights, zero gradients
     }
@@ -332,8 +356,45 @@ extern "C" int hbr_composite_fwd(const float* t, int64_t t_rs, const float* rgb,
   if (int rc = check_composite(t, t_rs, rgb, sigma, R, S)) return rc;
   HBR_REQUIRE(C != nullptr, "C is NULL");
   if (!(ert_tau > 0.f)) ert_tau = 3.0e38f;                           // <= 0 / NaN: off (no fp32 optical depth exceeds it)
-  composite_fwd_kernel<<<(unsigned)ceil_div(R, kRaysPerCta), kRaysPerCta * 32, 0, as_stream(stream)>>>(
-      t, t_rs, rgb, rgb_st, sigma, sig_st, dn, dn_scalar, mask, rowmap, R, (int)S, C, w, ert_tau);
+  composite_fwd_kernel<false><<<(unsigned)ceil_div(R, kRaysPerCta), kRaysPerCta * 32, 0, as_stream(stream)>>>(
+      t, t_rs, rgb, rgb_st, sigma, sig_st, dn, dn_scalar, mask, rowmap, R, (int)S, C, w, ert_tau, nullptr, nullptr);
+  HBR_LAUNCH_CHECK();
+  return HBR_OK;
+}
+
+extern "C" int hbr_composite_maps_fwd(const float* t, int64_t t_rs, const float* rgb, int64_t rgb_st, const float* sigma,
+                                      int64_t sig_st, const float* dn, float dn_scalar, const uint8_t* mask,
+                                      const int32_t* rowmap, int64_t R, int64_t S, float* C, float* w, float* depth,
+                                      float* opacity, float ert_tau, void* stream) {
+  if (R == 0) return HBR_OK;
+  if (int rc = check_composite(t, t_rs, rgb, sigma, R, S)) return rc;
+  HBR_REQUIRE(C != nullptr, "C is NULL");
+  if (!(ert_tau > 0.f)) ert_tau = 3.0e38f;
+  composite_fwd_kernel<true><<<(unsigned)ceil_div(R, kRaysPerCta), kRaysPerCta * 32, 0, as_stream(stream)>>>(
+      t, t_rs, rgb, rgb_st, sigma, sig_st, dn, dn_scalar, mask, rowmap, R, (int)S, C, w, ert_tau, depth, opacity);
+  HBR_LAUNCH_CHECK();
+  return HBR_OK;
+}
+
+template <bool MAPS>
+static int composite_bwd_launch(const float* t, int64_t t_rs, const float* rgb, int64_t rgb_st, const float* sigma,
+                                int64_t sig_st, const float* dn, float dn_scalar, const uint8_t* mask, const int32_t* rowmap,
+                                int64_t R, int64_t S, const float* gC, const float* gD, const float* gA, float* drgb,
+                                int64_t drgb_st, float* dsig, int64_t dsig_st, float ert_tau, void* stream) {
+  if (!(ert_tau > 0.f)) ert_tau = 3.0e38f;
+  if (drgb_st == 4 && dsig_st == 4 && dsig == drgb + 3)
+    HBR_REQUIRE((uintptr_t)drgb % 16 == 0, "packed gradient buffer must be 16-byte aligned");
+  const unsigned grid = (unsigned)ceil_div(R, kRaysPerCta);
+  cudaStream_t st = as_stream(stream);
+#define HBR_CB(N)                                                                                                      \
+  composite_bwd_kernel<N, MAPS><<<grid, kRaysPerCta * 32, 0, st>>>(t, t_rs, rgb, rgb_st, sigma, sig_st, dn, dn_scalar, \
+                                                                   mask, rowmap, R, (int)S, gC, drgb, drgb_st, dsig,   \
+                                                                   dsig_st, ert_tau, gD, gA)
+  if (S <= 128) HBR_CB(4);
+  else if (S <= 256) HBR_CB(8);
+  else if (S <= 512) HBR_CB(16);
+  else HBR_CB(32);
+#undef HBR_CB
   HBR_LAUNCH_CHECK();
   return HBR_OK;
 }
@@ -345,21 +406,20 @@ extern "C" int hbr_composite_bwd(const float* t, int64_t t_rs, const float* rgb,
   if (R == 0) return HBR_OK;
   if (int rc = check_composite(t, t_rs, rgb, sigma, R, S)) return rc;
   HBR_REQUIRE(gC && drgb && dsig, "NULL pointer");
-  if (!(ert_tau > 0.f)) ert_tau = 3.0e38f;
-  if (drgb_st == 4 && dsig_st == 4 && dsig == drgb + 3)
-    HBR_REQUIRE((uintptr_t)drgb % 16 == 0, "packed gradient buffer must be 16-byte aligned");
-  const unsigned grid = (unsigned)ceil_div(R, kRaysPerCta);
-  cudaStream_t st = as_stream(stream);
-#define HBR_CB(N)                                                                                               \
-  composite_bwd_kernel<N><<<grid, kRaysPerCta * 32, 0, st>>>(t, t_rs, rgb, rgb_st, sigma, sig_st, dn, dn_scalar, \
-                                                             mask, rowmap, R, (int)S, gC, drgb, drgb_st, dsig, dsig_st, ert_tau)
-  if (S <= 128) HBR_CB(4);
-  else if (S <= 256) HBR_CB(8);
-  else if (S <= 512) HBR_CB(16);
-  else HBR_CB(32);
-#undef HBR_CB
-  HBR_LAUNCH_CHECK();
-  return HBR_OK;
+  return composite_bwd_launch<false>(t, t_rs, rgb, rgb_st, sigma, sig_st, dn, dn_scalar, mask, rowmap, R, S, gC, nullptr,
+                                     nullptr, drgb, drgb_st, dsig, dsig_st, ert_tau, stream);
+}
+
+extern "C" int hbr_composite_maps_bwd(const float* t, int64_t t_rs, const float* rgb, int64_t rgb_st, const float* sigma,
+                                      int64_t sig_st, const float* dn, float dn_scalar, const uint8_t* mask,
+                                      const int32_t* rowmap, int64_t R, int64_t S, const float* gC, const float* gD,
+                                      const float* gA, float* drgb, int64_t drgb_st, float* dsig, int64_t dsig_st,
+                                      float ert_tau, void* stream) {
+  if (R == 0) return HBR_OK;
+  if (int rc = check_composite(t, t_rs, rgb, sigma, R, S)) return rc;
+  HBR_REQUIRE(drgb && dsig, "NULL pointer");
+  return composite_bwd_launch<true>(t, t_rs, rgb, rgb_st, sigma, sig_st, dn, dn_scalar, mask, rowmap, R, S, gC, gD, gA,
+                                    drgb, drgb_st, dsig, dsig_st, ert_tau, stream);
 }
 
 extern "C" int hbr_hier_sample(float* w, const float* t, const float* u, const float* cand, int64_t R, int64_t S,

@@ -185,4 +185,9 @@ class HashEncoder(nn.Module):
         table = self._flat_table()
         if table.device != x.device:
             raise RuntimeError(f"encoder tables are on {table.device}, x on {x.device}")
-        return _HashEncodeFn.apply(x.detach(), self, *[e.weight for e in self.Embedding_list])
+        weights = [e.weight for e in self.Embedding_list]
+        if not torch.is_grad_enabled():
+            # needs_input_grad follows requires_grad, not the grad mode: under no_grad the node would still zero a table
+            # gradient buffer that no backward ever reads
+            weights = [w.detach() for w in weights]
+        return _HashEncodeFn.apply(x.detach(), self, *weights)

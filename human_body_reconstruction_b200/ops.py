@@ -328,6 +328,30 @@ def composite_bwd(t, rgb, rgb_stride, sigma, sigma_stride, dir_norm, mask, R, S,
                                   float(ert_tau), stream()))
 
 
+def composite_maps_fwd(t, rgb, rgb_stride, sigma, sigma_stride, dir_norm, mask, R, S, want_w=True, ert_tau=0.0, rowmap=None,
+                       want_depth=True, want_opacity=True):
+    """composite_fwd plus the per-ray maps depth = sum w t (units of t; z-depth = depth / dir_norm) and opacity = sum w, in
+    the same kernel.  Returns (C (R,3), w (R,S) or None, depth (R) or None, opacity (R) or None)."""
+    dn, dns = _dn_args(dir_norm, R, t.device)
+    Cc = torch.empty((R, 3), device=t.device, dtype=torch.float32)
+    w = torch.empty((R, S), device=t.device, dtype=torch.float32) if want_w else None
+    D = torch.empty((R,), device=t.device, dtype=torch.float32) if want_depth else None
+    A = torch.empty((R,), device=t.device, dtype=torch.float32) if want_opacity else None
+    check(lib().hbr_composite_maps_fwd(ptr(t), 0 if t.dim() == 1 else S, ptr(rgb), rgb_stride, ptr(sigma), sigma_stride,
+                                       ptr(dn), dns, ptr(mask), ptr(rowmap), R, S, ptr(Cc), ptr(w), ptr(D), ptr(A),
+                                       float(ert_tau), stream()))
+    return Cc, w, D, A
+
+
+def composite_maps_bwd(t, rgb, rgb_stride, sigma, sigma_stride, dir_norm, mask, R, S, gC, gD, gA, drgb, drgb_stride, dsig,
+                       dsig_stride, ert_tau=0.0, rowmap=None):
+    """composite_bwd with the gradients gD, gA (R) of the depth and opacity maps; any of gC, gD, gA may be None (= 0)."""
+    dn, dns = _dn_args(dir_norm, R, t.device)
+    check(lib().hbr_composite_maps_bwd(ptr(t), 0 if t.dim() == 1 else S, ptr(rgb), rgb_stride, ptr(sigma), sigma_stride,
+                                       ptr(dn), dns, ptr(mask), ptr(rowmap), R, S, ptr(gC), ptr(gD), ptr(gA), ptr(drgb),
+                                       drgb_stride, ptr(dsig), dsig_stride, float(ert_tau), stream()))
+
+
 class CompositePacked(torch.autograd.Function):
     """calc_color on the MLP's packed (R*S,4) [rgb,sigma] output -> (C (R,3), w (R,S)); w carries no gradient."""
 
@@ -354,6 +378,40 @@ class CompositePacked(torch.autograd.Function):
         d4 = torch.empty_like(out4)
         composite_bwd(t, out4, 4, out4[:, 3:], 4, dn, mask, R, S, _f32c(gC), d4, 4, d4[:, 3:], 4, ert_tau=ctx.ert_tau,
                       rowmap=ctx.rowmap)
+        return d4, None, None, None, None, None, None, None
+
+
+class CompositeMapsPacked(torch.autograd.Function):
+    """CompositePacked with the depth and opacity maps: out4 (R*S,4) [rgb, sigma] (or a compacted list read through rowmap)
+    -> (C (R,3), w (R,S), depth (R), opacity (R)).  C, depth and opacity carry gradients, w does not.  depth = sum_s w_s t_s
+    is the distance along the unit ray direction (z-depth = depth / dir_norm), opacity = sum_s w_s; neither is normalised
+    or clamped."""
+
+    @staticmethod
+    def forward(ctx, out4, t, dir_norm, mask, R, S, ert_tau=0.0, rowmap=None):
+        require_cuda(out4, t)
+        out4 = _f32c(out4)
+        t = _f32c(t)
+        ctx.ert_tau = float(ert_tau)
+        Cc, w, D, A = composite_maps_fwd(t, out4, 4, out4[:, 3:], 4, dir_norm, mask, R, S, ert_tau=ert_tau, rowmap=rowmap)
+        ctx.rowmap = rowmap
+        ctx.save_for_backward(out4, t, dir_norm if torch.is_tensor(dir_norm) else None, mask)
+        ctx.dn_scalar = None if torch.is_tensor(dir_norm) else dir_norm
+        ctx.RS = (R, S)
+        ctx.mark_non_differentiable(w)
+        ctx.set_materialize_grads(False)          # an unused map costs no zero-filled gradient: the kernel reads NULL as 0
+        return Cc, w, D, A
+
+    @staticmethod
+    def backward(ctx, gC, _gw, gD, gA):
+        if gC is None and gD is None and gA is None:
+            return (None,) * 8
+        out4, t, dn, mask = ctx.saved_tensors
+        dn = dn if dn is not None else ctx.dn_scalar
+        R, S = ctx.RS
+        d4 = torch.empty_like(out4)
+        composite_maps_bwd(t, out4, 4, out4[:, 3:], 4, dn, mask, R, S, _f32c(gC), _f32c(gD), _f32c(gA), d4, 4, d4[:, 3:], 4,
+                           ert_tau=ctx.ert_tau, rowmap=ctx.rowmap)
         return d4, None, None, None, None, None, None, None
 
 

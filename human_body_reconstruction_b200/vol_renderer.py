@@ -12,6 +12,7 @@ The legacy classic-NeRF MLP class (vol_renderer.py:12-86) is not part of the hot
 from __future__ import annotations
 
 import os
+from collections import namedtuple
 from typing import Optional, Tuple
 
 import torch
@@ -310,6 +311,18 @@ def _side_stream(device) -> torch.cuda.Stream:
     return s
 
 
+def _field_params(enc, mlp):
+    """The parameters a field autograd node depends on.  Under no_grad they are passed detached: the nodes decide from
+    needs_input_grad (which follows requires_grad, not the grad mode) whether to allocate and zero a table gradient buffer
+    in their forward, and no backward would ever read it."""
+    ps = [*[e.weight for e in enc.Embedding_list], *mlp._ordered()]
+    return ps if torch.is_grad_enabled() else [p.detach() for p in ps]
+
+
+# Volume_Renderer.render: colours, depth and opacity maps of the coarse and the fine pass, the eikonal norms (SDF mode)
+RenderOut = namedtuple("RenderOut", "rgb_coarse rgb_fine depth_coarse depth_fine opacity_coarse opacity_fine norm")
+
+
 def _unwrap(model):
     if isinstance(model, nn.DataParallel) and len(model.device_ids) <= 1:
         return model.module
@@ -467,8 +480,14 @@ class Volume_Renderer:
         width = enc.L * enc.F + enc.E
         return width == mlp._in0 and (width % 2 == 0) and ((width == 32 and mlp.d_view <= 25) or width == 64)
 
-    def _field_pass(self, mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed):
-        """positions -> encoder -> MLP -> compositing for depths t ((S,) shared or (R,S) per ray)."""
+    def _composite(self, out4, t, dir_norm, mask, R, S, rowmap=None, maps=False):
+        if maps:
+            return ops.CompositeMapsPacked.apply(out4, t, dir_norm, mask, R, S, self._ert_tau(), rowmap)
+        return ops.CompositePacked.apply(out4, t, dir_norm, mask, R, S, self._ert_tau(), rowmap)
+
+    def _field_pass(self, mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed, maps=False):
+        """positions -> encoder -> MLP -> compositing for depths t ((S,) shared or (R,S) per ray) -> (C, w), or with maps
+        (C, w, depth, opacity)."""
         R, S = rays_o.shape[0], t.shape[-1]
         if not self._can_fuse(mlp) and self._can_chain(mlp):
             enc = self.Pos_encode
@@ -477,25 +496,23 @@ class Volume_Renderer:
             if mask_needed and self.compact and S <= 1024 and R * S < 2 ** 31:
                 mu, sig = self._norm_host()
                 out4, rowmap, _ = _FieldCompactFn.apply(rays_o, rays_d, t.float().contiguous(), dir_enc.float().contiguous(),
-                                                        self.bool_grid, mu, sig, enc, mlp,
-                                                        *[e.weight for e in enc.Embedding_list], *mlp._ordered())
-                return ops.CompositePacked.apply(out4, t, dir_norm, None, R, S, self._ert_tau(), rowmap)
+                                                        self.bool_grid, mu, sig, enc, mlp, *_field_params(enc, mlp))
+                return self._composite(out4, t, dir_norm, None, R, S, rowmap, maps)
             mask = self.get_mask(ops.ray_points(rays_o, rays_d, t).view(-1, 3)) if mask_needed else None
             out4 = _FieldRaysFn.apply(rays_o, rays_d, t.float().contiguous(), dir_enc.float().contiguous(), enc, mlp,
-                                      *[e.weight for e in enc.Embedding_list], *mlp._ordered())
-            return ops.CompositePacked.apply(out4, t, dir_norm, mask, R, S, self._ert_tau())
+                                      *_field_params(enc, mlp))
+            return self._composite(out4, t, dir_norm, mask, R, S, None, maps)
         pts = ops.ray_points(rays_o, rays_d, t).view(-1, 3)
         mask = self.get_mask(pts) if mask_needed else None
         if self._can_fuse(mlp):
             enc = self.Pos_encode
             if enc._flat_table().device != pts.device:
                 raise RuntimeError(f"encoder tables are on {enc._flat_table().device}, rays on {pts.device}")
-            out4 = _FieldFn.apply(pts, dir_enc, S, enc, mlp, *[e.weight for e in enc.Embedding_list], *mlp._ordered())
+            out4 = _FieldFn.apply(pts, dir_enc, S, enc, mlp, *_field_params(enc, mlp))
         else:
             feat = self.Pos_encode(pts)
             out4 = mlp.field(feat, dir_enc, S)
-        Cc, w = ops.CompositePacked.apply(out4, t, dir_norm, mask, R, S, self._ert_tau())
-        return Cc, w
+        return self._composite(out4, t, dir_norm, mask, R, S, None, maps)
 
     def vol_render(self, model, rays_d: torch.Tensor, rays_o: torch.Tensor, num_samples=100,
                    t: Optional[torch.Tensor] = None, update_mask=False, dir_norm=1, hierarchical=True,
@@ -549,6 +566,90 @@ class Volume_Renderer:
         Cr, Cf = self._render_rays(mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed, hierarchical, _u, _u_cand)
         return Cr, Cf, None
 
+    def render(self, model, rays_d: torch.Tensor, rays_o: torch.Tensor, num_samples=100, t: Optional[torch.Tensor] = None,
+               dir_norm=1, hierarchical=True) -> RenderOut:
+        """vol_render with depth and opacity maps: RenderOut(rgb_coarse, rgb_fine, depth_coarse, depth_fine, opacity_coarse,
+        opacity_fine, norm).  Same RNG draws, routes (chained, fused, compact, masked, early ray termination) and ray chunks
+        as vol_render(update_mask=False), so the colours are bit-identical to vol_render's; without hierarchical the fine
+        outputs are the coarse ones.
+          depth = sum_s w_s t_s: distance along the unit ray direction, in the units of t (p = o + d t, |d| = 1 as get_od
+                  and ops.ray_gen return it).  z-depth along the camera axis is depth / dir_norm.
+          opacity = sum_s w_s: what a person-mask loss supervises.
+        Neither is normalised by the opacity or clamped: MLP_3D's LeakyReLU density can be slightly negative, so weights and
+        opacity can leave [0, 1].  Both carry gradients (to the tables and the MLP through the compositor's backward).
+        Native modules only: the NeRF route (HashEncoder / PositionalEncoder / MLP_3D) and the native SDF route
+        (hierarchical=False, reference VarModel; norm = eikonal norms, maps from the SDF weights); anything else raises
+        TypeError."""
+        if not rays_d.is_cuda:
+            raise RuntimeError("Volume_Renderer.render needs CUDA tensors (there is no CPU fallback)")
+        if t is None:
+            t = strat_sampler(self.near, self.far, num_samples, device=rays_d.device)                 # RNG draw #1
+        if self.use_sdf:
+            sdf_mlp = self._native_sdf(model) if (self.sdf_native and hierarchical is not True and t.shape[-1] <= 1024) else None
+            if sdf_mlp is None or not self._grid_all_true():
+                raise TypeError("Volume_Renderer.render in SDF mode needs the native SDF route: HashEncoder / "
+                                "PositionalEncoder / MLP_3D with the reference's VarModel, hierarchical=False, at most 1024 "
+                                "samples and an all-True occupancy grid")
+            self._auto_dp(sdf_mlp)
+            Cr, w, norm = self._sdf_pass(sdf_mlp, rays_o, rays_d, t)
+            D, A = (w * t).sum(-1), w.sum(-1)
+            return RenderOut(Cr, Cr, D, D, A, A, norm)
+        mlp = self._native(model)
+        if mlp is None:
+            raise TypeError("Volume_Renderer.render needs the native HashEncoder / PositionalEncoder / MLP_3D")
+        self._auto_dp(mlp)
+        rays_o = rays_o.float().contiguous()
+        rays_d = rays_d.float().contiguous()
+        dir_enc = self.Dir_encode(rays_d)
+        mask_needed = not self._grid_all_true()
+        R, S = rays_o.shape[0], t.shape[-1]
+        per = max(1, int(self.max_points) // (S * (3 if hierarchical is True else 1)))
+        if R > per:
+            _u = _u_cand = None
+            if hierarchical is True:                                        # drawn once for the batch, as vol_render does
+                _u = torch.rand((R, S), device=rays_o.device)                                  # RNG draw #2
+                _u_cand = torch.rand(S, device=rays_o.device)                                  # RNG draw #3
+            dn_rows = torch.is_tensor(dir_norm) and dir_norm.numel() == R
+            parts = []
+            for r0 in range(0, R, per):
+                sl = slice(r0, min(R, r0 + per))
+                parts.append(self._render_rays(mlp, rays_o[sl], rays_d[sl], t, dir_enc[sl], dir_norm[sl] if dn_rows else dir_norm,
+                                               mask_needed, hierarchical, _u[sl] if _u is not None else None, _u_cand, maps=True))
+            out = [torch.cat(c) for c in zip(*parts)]
+            return RenderOut(*out, None)
+        return RenderOut(*self._render_rays(mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed, hierarchical, None, None,
+                                            maps=True), None)
+
+    @torch.no_grad()
+    def render_view(self, model, c2w, num_samples, hierarchical=True, chunk=1 << 16, t: Optional[torch.Tensor] = None):
+        """Whole views from camera poses: c2w (4,4) or (V,4,4), the renderer's H, W, K.  Rays are generated on the device
+        (ops.ray_gen) chunk by chunk -- `chunk` rays at a time, never V*H*W at once -- and each chunk is one render() call
+        (dir_norm = the ray generator's direction norm).  Returns rgb (V,H,W,3) (the fine colour when hierarchical), depth
+        (V,H,W) and opacity (V,H,W), from the fine pass when hierarchical.  Runs under no_grad; without `t` every chunk
+        draws its own stratified depths, so the result depends on `chunk` exactly as the RNG stream does."""
+        dev = self.bool_grid.device
+        if dev.type != "cuda":
+            raise RuntimeError("Volume_Renderer.render_view needs a CUDA device (there is no CPU fallback)")
+        c2w = torch.as_tensor(c2w).to(dev, torch.float32)
+        if c2w.dim() == 2:
+            c2w = c2w[None]
+        if c2w.shape[1:] != (4, 4):
+            raise ValueError("c2w must be (4,4) or (V,4,4)")
+        V, H, W = c2w.shape[0], int(self.H), int(self.W)
+        n = V * H * W
+        chunk = max(1, int(chunk))
+        rgb = torch.empty((n, 3), device=dev, dtype=torch.float32)
+        depth = torch.empty((n,), device=dev, dtype=torch.float32)
+        opacity = torch.empty((n,), device=dev, dtype=torch.float32)
+        for first in range(0, n, chunk):
+            m = min(chunk, n - first)
+            o, d, nrm, _ = ops.ray_gen(c2w, H, W, self.K, first=first, n_rays=m)
+            out = self.render(model, d, o, num_samples, t=t, dir_norm=nrm, hierarchical=hierarchical)
+            rgb[first:first + m] = out.rgb_fine
+            depth[first:first + m] = out.depth_fine
+            opacity[first:first + m] = out.opacity_fine
+        return rgb.view(V, H, W, 3), depth.view(V, H, W), opacity.view(V, H, W)
+
     def _auto_dp(self, mlp):
         """launch_rank.py's zero-edit multi-GPU run of the trainer (HBR_AUTO_DP=1): at the first native render of a process
         that belongs to a process group, take rank 0's parameters and attach the gradient exchange (dist.auto_attach);
@@ -574,6 +675,11 @@ class Volume_Renderer:
         the density head's LeakyReLU value in column 3), then hbr_composite_sdf_* forms 2*sigmoid - 1 and composites in one
         kernel each way, and the eikonal norms come from the 6-point stencil (MLP_3D.eikonal_norms).  dir_norm plays no
         part (helper.py:71 computes del_t, the SDF branch never reads it).  Returns (Cr, Cr, norm) like the reference."""
+        Cr, _, norm = self._sdf_pass(mlp, rays_o, rays_d, t)
+        return Cr, Cr, norm
+
+    def _sdf_pass(self, mlp, rays_o, rays_d, t):
+        """_render_sdf's pass -> (Cr, w (R,S) with a gradient, eikonal norms)."""
         rays_o = rays_o.float().contiguous()
         rays_d = rays_d.float().contiguous()
         dir_enc = self.Dir_encode(rays_d)
@@ -582,22 +688,26 @@ class Volume_Renderer:
         pts = ops.ray_points(rays_o, rays_d, t).view(-1, 3)
         if self._can_chain(mlp):
             out4 = _FieldRaysFn.apply(rays_o, rays_d, t.float().contiguous(), dir_enc.float().contiguous(), enc, mlp,
-                                      *[e.weight for e in enc.Embedding_list], *mlp._ordered())
+                                      *_field_params(enc, mlp))
         else:
             out4 = mlp.field(enc(pts), dir_enc, S, raw=True)
-        Cr, _ = ops.CompositeSdfPacked.apply(out4, self.var_model.b, R, S, bool(mlp.use_sdf))
+        Cr, w = ops.CompositeSdfPacked.apply(out4, self.var_model.b, R, S, bool(mlp.use_sdf))
         norm = mlp.eikonal_norms(pts, encoder=enc)
-        return Cr, Cr, norm
+        return Cr, w, norm
 
-    def _render_rays(self, mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed, hierarchical, _u, _u_cand):
-        Cr, w = self._field_pass(mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed)
+    def _render_rays(self, mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed, hierarchical, _u, _u_cand, maps=False):
+        """-> (Cr, Cf), or with maps (Cr, Cf, depth_r, depth_f, opacity_r, opacity_f)."""
+        coarse = self._field_pass(mlp, rays_o, rays_d, t, dir_enc, dir_norm, mask_needed, maps)
+        Cr, w = coarse[0], coarse[1]
         if hierarchical is True:
             _, t_fine = hierarchical_sampling(rays_o, rays_d, z_vals=t, weights=w, n_samples=t.shape[-1], tn=self.near,
                                               tf=self.far, device="cuda", _u=_u, _u_cand=_u_cand)   # RNG draws #2, #3
-            Cf, _ = self._field_pass(mlp, rays_o, rays_d, t_fine, dir_enc, dir_norm, False)    # the fine pass never masks (:237)
+            fine = self._field_pass(mlp, rays_o, rays_d, t_fine, dir_enc, dir_norm, False, maps)  # the fine pass never masks (:237)
         else:
-            Cf = Cr
-        return Cr, Cf
+            fine = coarse
+        if maps:
+            return Cr, fine[0], coarse[2], fine[2], coarse[3], fine[3]
+        return Cr, fine[0]
 
     def _generic(self, model, rays_d, rays_o, t, update_mask, dir_norm, hierarchical, _u, _u_cand):
         """Reference data flow for foreign encoders / models (vol_renderer.py:165-245)."""

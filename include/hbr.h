@@ -279,6 +279,24 @@ int hbr_composite_bwd(const float* t, int64_t t_ray_stride, const float* rgb, in
                       const uint8_t* mask, const int32_t* rowmap, int64_t R, int64_t S, const float* gC,
                       float* drgb, int64_t drgb_stride, float* dsigma, int64_t dsigma_stride, float ert_tau,
                       void* stream);
+/* The same compositor with per-ray depth and opacity maps, formed in the same pass from the same weights:
+ *   depth (R) = sum_s w_s t_s   -- distance along the unit ray direction, in the units of t (p = o + d t with |d| = 1);
+ *                                 z-depth is depth / dir_norm.  Not normalised by the opacity, not clamped.
+ *   opacity (R) = sum_s w_s     -- w may be negative (LeakyReLU density), so opacity can leave [0, 1] like the weights.
+ * Either map may be NULL (not written).  Every input form of hbr_composite_fwd is accepted (shared / per-ray t, dir_norm
+ * tensor or scalar, mask, rowmap, ert_tau: skipped chunks contribute 0); C and w are bit-identical to hbr_composite_fwd's.
+ * bwd: gD, gA (R) are the gradients of depth and opacity (NULL = 0; gC may be NULL too); the per-sample term of the
+ * closed-form backward becomes c_s = gC.rgb_s + gD t_s + gA, d(rgb) = w gC is unchanged.  With gD = gA = 0 the gradients
+ * equal hbr_composite_bwd's.  One kernel per call, the colour-only kernels with the map code compiled in. */
+int hbr_composite_maps_fwd(const float* t, int64_t t_ray_stride, const float* rgb, int64_t rgb_stride,
+                           const float* sigma, int64_t sigma_stride, const float* dir_norm, float dir_norm_scalar,
+                           const uint8_t* mask, const int32_t* rowmap, int64_t R, int64_t S, float* C, float* w,
+                           float* depth, float* opacity, float ert_tau, void* stream);
+int hbr_composite_maps_bwd(const float* t, int64_t t_ray_stride, const float* rgb, int64_t rgb_stride,
+                           const float* sigma, int64_t sigma_stride, const float* dir_norm, float dir_norm_scalar,
+                           const uint8_t* mask, const int32_t* rowmap, int64_t R, int64_t S, const float* gC,
+                           const float* gD, const float* gA, float* drgb, int64_t drgb_stride, float* dsigma,
+                           int64_t dsigma_stride, float ert_tau, void* stream);
 
 /* ---- a11: hierarchical_sampling, helper.py:23-51 --------------------------------------------------
  * w (R,S) coarse weights (negatives treated as 0; written back clamped when clamp_in_place != 0,
