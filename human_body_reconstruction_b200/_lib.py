@@ -143,6 +143,7 @@ SIGNATURES = {
     "hbr_mlp_act_floats": ([], _i64),
     "hbr_hash_encode_fwd": ([_vp, _i32, _i64, _vp, _geom_p, _vp, _i64, _vp], C.c_int),
     "hbr_hash_encode_bwd": ([_vp, _i32, _i64, _vp, _i64, _geom_p, _vp, _i32, _i32, _vp], C.c_int),
+    "hbr_hash_encode_dx": ([_vp, _i32, _i64, _vp, _geom_p, _vp, _i64, _vp, _vp], C.c_int),
     "hbr_hash_indices": ([_vp, _i32, _i64, _geom_p, _vp, _vp, _vp], C.c_int),
     "hbr_dir_encode": ([_vp, _i32, _i64, _i32, _i32, _vp, _vp], C.c_int),
     "hbr_mlp_fwd_f32": ([_vp, _i64, _vp, _i64, _i64, _vp, _dims_p, _vp, _vp, _vp], C.c_int),
@@ -230,7 +231,7 @@ DEBUG_SIGNATURES = {
 
 # kernels launched by one call of each entry point (for bench.py's gpu_launches claim)
 KERNELS_PER_CALL = {
-    "hbr_hash_encode_fwd": 1, "hbr_hash_encode_bwd": 1, "hbr_hash_encode_fwd_rays": 1, "hbr_hash_encode_bwd_rays": 1, "hbr_hash_indices": 1, "hbr_dir_encode": 1,
+    "hbr_hash_encode_fwd": 1, "hbr_hash_encode_bwd": 1, "hbr_hash_encode_dx": 1, "hbr_hash_encode_fwd_rays": 1, "hbr_hash_encode_bwd_rays": 1, "hbr_hash_indices": 1, "hbr_dir_encode": 1,
     "hbr_mlp_fwd_f32": 1, "hbr_mlp_bwd_f32": 2, "hbr_mlp_fwd_tc": 2, "hbr_mlp_bwd_tc": 3, "hbr_field_fwd_tc": 2, "hbr_field_bwd_tc": 3, "hbr_field_bwd_rays_tc": 3, "hbr_field_fwd_rays_tc": 1, "hbr_adam_step": 1, "hbr_adam_tick": 1, "hbr_adam_step_dev": 1, "hbr_allreduce_peer": 1, "hbr_allreduce_peer_stream": 1, "hbr_hash_encode_bwd_stream": 1, "hbr_hash_encode_bwd_rays_stream": 1, "hbr_hash_encode_bwd_lm": 1, "hbr_hash_encode_bwd_rays_lm": 1, "hbr_ray_gen": 1, "hbr_ray_bbox": 1, "hbr_ray_points": 1, "hbr_occupancy_mask": 1, "hbr_occupancy_update": 2, "hbr_compact_samples": 1, "hbr_hash_encode_fwd_pts": 1, "hbr_hash_encode_bwd_pts": 1,
     "hbr_composite_fwd": 1, "hbr_composite_bwd": 1, "hbr_composite_maps_fwd": 1, "hbr_composite_maps_bwd": 1, "hbr_strat_depths": 1, "hbr_mse_pair_fwd": 1, "hbr_mse_pair_bwd": 1, "hbr_mlp_tc_prepare": 1, "hbr_mlp_tc_reduce_grads": 1, "hbr_hier_sample": 1, "hbr_grid_points": 1,
     "hbr_composite_sdf_fwd": 1, "hbr_composite_sdf_bwd": 1, "hbr_sdf_stencil_points": 1, "hbr_sdf_eikonal_fwd": 1, "hbr_sdf_eikonal_bwd": 1,

@@ -480,6 +480,81 @@ __global__ void hash_idx_kernel(const XT* __restrict__ x, long long n, int32_t* 
   }
 }
 
+// ---- input gradient: dL/dx ---------------------------------------------------------------------------------
+// The forward's mapping and gathers, with the feature gradient dy in place of the output: per level the 8 corner rows are
+// contracted with dy (g_c = sum_f dy[lF+f] v_c[f]) and differentiated through the trilinear weights.  The cells and fracs
+// come from the same cell_of pipeline; the truncation toward zero has slope 1 on both sides of 0, so d(frac)/du = 1 and
+//   dL/du_x = sum_c g_c (bit_x(c) ? +1 : -1) wy wz   (y, z alike),   dx_a = sum_l (s_l / sigma) dL/du_a.
+// Each of the two threads of a point sums its own levels in order; the odd-level thread leaves its partial sum in shared
+// memory and the even-level thread adds it: a fixed order, no atomics, bitwise reproducible.  dx is overwritten.
+template <int F, bool POW2, typename XT, int UNR = 4>
+__global__ void __launch_bounds__(kHashThreads)
+hash_dx_kernel(const XT* __restrict__ x, long long n, const float* __restrict__ table, const float* __restrict__ dy,
+               long long dy_stride, float* __restrict__ dx, const __grid_constant__ HashGeom g) {
+  extern __shared__ float tile[];                    // [kTilePts][pitch] rows of dy, then [kTilePts][3] odd-level partials
+  const int C = g.L * F;
+  const int pitch = C | 1;
+  float* part = tile + kTilePts * pitch;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long base = (long long)blockIdx.x * kTilePts;
+  for (int r = warp; r < kTilePts; r += kHashThreads / 32) {
+    const long long gp = base + r;
+    for (int c = lane; c < C; c += 32) tile[r * pitch + c] = gp < n ? __ldg(dy + gp * dy_stride + c) : 0.f;
+  }
+  const int p = threadIdx.x & (kTilePts - 1);
+  const int grp = threadIdx.x / kTilePts;
+  float pt[3];
+  load_point(x, base + p, n, pt);
+  __syncthreads();
+
+  float acc[3] = {0.f, 0.f, 0.f};
+#pragma unroll UNR
+  for (int l = grp; l < g.L; l += 2) {
+    const float s = g.scale[l];
+    long long ix, iy, iz;
+    float fx, fy, fz;
+    cell_of(pt[0], g.mu[0], g.sigma, s, ix, fx);
+    cell_of(pt[1], g.mu[1], g.sigma, s, iy, fy);
+    cell_of(pt[2], g.mu[2], g.sigma, s, iz, fz);
+    uint32_t idx[8];
+    corner_indices<POW2>(ix, iy, iz, g.T, idx);
+    const float* lvl = table + (size_t)l * g.T * F;
+    float v[8][F];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) load_feat<F>(lvl, idx[c], v[c]);          // 8 independent gathers in flight
+    float gc[8];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+      gc[c] = 0.f;
+#pragma unroll
+      for (int f = 0; f < F; ++f) gc[c] = fmaf(tile[p * pitch + l * F + f], v[c][f], gc[c]);
+    }
+    const float wx[2] = {1.f - fx, fx}, wy[2] = {1.f - fy, fy}, wz[2] = {1.f - fz, fz};
+    float du[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+      const int bx = c & 1, by = (c >> 1) & 1, bz = (c >> 2) & 1;
+      const float sg = bx ? gc[c] : -gc[c], sy = by ? gc[c] : -gc[c], sz = bz ? gc[c] : -gc[c];
+      du[0] = fmaf(sg, wy[by] * wz[bz], du[0]);
+      du[1] = fmaf(sy, wx[bx] * wz[bz], du[1]);
+      du[2] = fmaf(sz, wx[bx] * wy[by], du[2]);
+    }
+    const float k = s / g.sigma;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) acc[a] = fmaf(k, du[a], acc[a]);
+  }
+  if (grp == 1) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) part[p * 3 + a] = acc[a];
+  }
+  __syncthreads();
+  const long long gp = base + p;
+  if (grp == 0 && gp < n) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) dx[gp * 3 + a] = acc[a] + part[p * 3 + a];
+  }
+}
+
 static int check_geom(const hbr_hash_geom* g) {
   HBR_REQUIRE(g != nullptr, "geom is NULL");
   HBR_REQUIRE(g->L >= 1 && g->L <= HBR_MAX_LEVELS, "L=%d out of range [1,%d]", g->L, HBR_MAX_LEVELS);
@@ -506,6 +581,16 @@ static int launch_bwd(const void* x, int64_t n, const float* dy, int64_t ds, con
   HBR_CUDA(cudaFuncSetAttribute(hash_bwd_kernel<F, POW2, XT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   hash_bwd_kernel<F, POW2, XT><<<(unsigned)ceil_div(n, kTilePts), kHashThreads, smem, st>>>(
       static_cast<const XT*>(x), n, dy, ds, dt, g, l0, l1, nullptr, ChunkPlan{});
+  HBR_LAUNCH_CHECK();
+  return HBR_OK;
+}
+template <int F, bool POW2, typename XT>
+static int launch_dx(const void* x, int64_t n, const float* table, const float* dy, int64_t ds, const HashGeom& g, float* dx,
+                     cudaStream_t st) {
+  const size_t smem = (size_t)kTilePts * (((g.L * F) | 1) + 3) * sizeof(float);
+  auto k = hash_dx_kernel<F, POW2, XT>;
+  HBR_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k<<<(unsigned)ceil_div(n, kTilePts), kHashThreads, smem, st>>>(static_cast<const XT*>(x), n, table, dy, ds, dx, g);
   HBR_LAUNCH_CHECK();
   return HBR_OK;
 }
@@ -639,6 +724,19 @@ extern "C" int hbr_hash_encode_bwd(const void* x, int x_dtype, int64_t n, const 
   if (level_begin == level_end) return HBR_OK;
   const HashGeom g = to_device_geom(*geom);
   HBR_DISPATCH_HASH(launch_bwd, x, n, dy, dy_stride, g, dtable, level_begin, level_end, as_stream(stream));
+}
+
+extern "C" int hbr_hash_encode_dx(const void* x, int x_dtype, int64_t n, const float* table, const hbr_hash_geom* geom,
+                                  const float* dy, int64_t dy_stride, float* dx, void* stream) {
+  if (int rc = check_geom(geom)) return rc;
+  HBR_REQUIRE(x_dtype == HBR_F32 || x_dtype == HBR_F16, "x_dtype %d", x_dtype);
+  HBR_REQUIRE(n >= 0 && n < (1LL << 40), "n=%lld", (long long)n);
+  if (n == 0) return HBR_OK;
+  HBR_REQUIRE(x && table && dy && dx, "NULL pointer");
+  HBR_REQUIRE(dy_stride >= geom->L * geom->F, "dy_stride %lld too small", (long long)dy_stride);
+  HBR_REQUIRE((uintptr_t)table % 16 == 0, "table must be 16-byte aligned");
+  const HashGeom g = to_device_geom(*geom);
+  HBR_DISPATCH_HASH(launch_dx, x, n, table, dy, dy_stride, g, dx, as_stream(stream));
 }
 
 extern "C" int hbr_hash_indices(const void* x, int x_dtype, int64_t n, const hbr_hash_geom* geom,

@@ -11,6 +11,7 @@ from __future__ import annotations
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import ops
 
@@ -23,6 +24,7 @@ class _HashEncodeFn(torch.autograd.Function):
         y = ops.hash_encode_fwd(x, table, geom)
         ctx.enc = enc
         ctx.geom = geom
+        ctx.table = table if ctx.needs_input_grad[0] else None     # the tables the positions' gradient is taken at
         ctx.save_for_backward(x)
         ctx.g = None
         if any(ctx.needs_input_grad[2:]):
@@ -33,11 +35,17 @@ class _HashEncodeFn(torch.autograd.Function):
         return y
 
     @staticmethod
+    @once_differentiable
     def backward(ctx, dy):
         (x,) = ctx.saved_tensors
         enc = ctx.enc
         L, T, F = enc.L, enc.T, enc.F
         dp = enc._dp
+        # HashEncoder.position_grad: dL/dx through the trilinear weights (first order only)
+        dx = ops.hash_encode_dx(x, ctx.table, ctx.geom, dy).to(x.dtype) if ctx.table is not None else None
+        ctx.table = None
+        if not any(ctx.needs_input_grad[2:]):       # positions only (frozen tables): no table gradient to form
+            return (dx, None) + (None,) * L
         if dp is not None:
             # Data-parallel run (dist._GradExchange): accumulate into the persistent buffer of this backward pass.  The
             # last table backward of the pass runs in level chunks and publishes each one as soon as its scatter-add is
@@ -51,12 +59,12 @@ class _HashEncodeFn(torch.autograd.Function):
                 ev_pre = torch.cuda.current_stream().record_event()
                 ops.hash_encode_bwd_stream(x, dy[:, : L * F], ctx.geom, g, plan, dp.done)
                 dp.exchange_streamed(plan, ops.hash_bwd_stream_tiles(x.shape[0]), after=(ev_pre,))
-                return (None, None) + (None,) * L
+                return (dx, None) + (None,) * L
             for l0, l1 in (dp.level_chunks(enc, L, x.shape[0]) if last else [(0, L)]):
                 ops.hash_encode_bwd(x, dy[:, : L * F], ctx.geom, g, l0, l1)
                 if last:
                     dp.publish(enc, g[l0:l1])
-            return (None, None) + (None,) * L
+            return (dx, None) + (None,) * L
         if ctx.g is not None:
             g, ev = ctx.g
             ctx.g = None
@@ -64,13 +72,21 @@ class _HashEncodeFn(torch.autograd.Function):
         else:
             g = torch.zeros((L, T, F), device=dy.device, dtype=torch.float32)
         ops.hash_encode_bwd(x, dy[:, : L * F], ctx.geom, g, 0, L)
-        # no gradient w.r.t. x: the interpolation weights are detached in the reference (hash_encoding.py:160)
-        return (None, None) + tuple(g[i] for i in range(L))
+        # no gradient w.r.t. x unless position_grad is set: the reference detaches the interpolation weights
+        # (hash_encoding.py:160)
+        return (dx, None) + tuple(g[i] for i in range(L))
 
 
 class HashEncoder(nn.Module):
     """hash_encoding.py:5-170.  Only dim == 3 has a CUDA implementation (dim == 2 serves the reference's
-    broken 2-D image demo, test_hash.py:108-205, which is out of scope)."""
+    broken 2-D image demo, test_hash.py:108-205, which is out of scope).
+
+    `position_grad` (default False, the reference's behaviour: positions are detached): when True and x.requires_grad,
+    forward keeps x in the graph and backward returns dL/dx from hbr_hash_encode_dx -- the trilinear weights
+    differentiated at the forward's cells, first order only (once_differentiable).  So
+    torch.autograd.grad(nerf(encoder(x))[:, 0].sum(), x) is the density's spatial gradient.  The fused ray routes of
+    Volume_Renderer form the sample positions inside their kernels and never call this forward: they have no position
+    gradient whatever the flag says."""
 
     def __init__(self, N_max, N_min, L, E=0, T=2 ** 14, F=2, dim=2, mu=None, sigma=None, device=None):
         super().__init__()
@@ -96,6 +112,7 @@ class HashEncoder(nn.Module):
         self._side = None
         self._dp = None               # the data-parallel gradient exchange attached to this module (dist._GradExchange)
         self._flat = None
+        self.position_grad = False    # see the class docstring
         self._reflatten()
 
     # -- flat storage ------------------------------------------------------------------------------------
@@ -190,4 +207,5 @@ class HashEncoder(nn.Module):
             # needs_input_grad follows requires_grad, not the grad mode: under no_grad the node would still zero a table
             # gradient buffer that no backward ever reads
             weights = [w.detach() for w in weights]
-        return _HashEncodeFn.apply(x.detach(), self, *weights)
+        keep = getattr(self, "position_grad", False) and x.requires_grad and torch.is_grad_enabled()
+        return _HashEncodeFn.apply(x if keep else x.detach(), self, *weights)

@@ -71,6 +71,18 @@ def hash_encode_bwd(x: torch.Tensor, dy: torch.Tensor, geom: HashGeom, dtable: t
                                     int(level_begin), int(level_end), stream()))
 
 
+def hash_encode_dx(x: torch.Tensor, table: torch.Tensor, geom: HashGeom, dy: torch.Tensor) -> torch.Tensor:
+    """dL/dx (n,3) fp32 for the feature gradient dy (n, >= L*F; columns past L*F are ignored).  Overwritten, not accumulated."""
+    require_cuda(x, table, dy)
+    x = x.contiguous()
+    if dy.dtype != torch.float32 or dy.stride(1) != 1:
+        dy = dy.float().contiguous()
+    n = x.shape[0]
+    dx = torch.empty((n, 3), device=x.device, dtype=torch.float32)
+    check(lib().hbr_hash_encode_dx(ptr(x), _xdtype(x), n, ptr(table), C.byref(geom), ptr(dy), dy.stride(0), ptr(dx), stream()))
+    return dx
+
+
 def _t_stride(t: torch.Tensor, S: int) -> int:
     return 0 if t.dim() == 1 else S
 

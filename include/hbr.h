@@ -76,6 +76,13 @@ int hbr_hash_encode_fwd(const void* x, int x_dtype, int64_t n, const float* tabl
 int hbr_hash_encode_bwd(const void* x, int x_dtype, int64_t n, const float* dy, int64_t dy_stride,
                         const hbr_hash_geom* geom_host, float* dtable, int level_begin, int level_end, void* stream);
 
+/* Gradient with respect to the POSITIONS (the reference detaches the interpolation weights and has none):
+ * dx (n,3) fp32 is OVERWRITTEN with dL/dx = sum_l (s_l/sigma) dL/du_l, the trilinear weights differentiated at the cells
+ * and fracs of the forward (truncation toward zero: d frac / du = 1).  dy: rows of dy_stride floats, the first L*F
+ * columns used (the E aux columns are ignored).  x fp32 or fp16.  Deterministic: no atomics. */
+int hbr_hash_encode_dx(const void* x, int x_dtype, int64_t n, const float* table, const hbr_hash_geom* geom_host,
+                       const float* dy, int64_t dy_stride, float* dx, void* stream);
+
 /* a2/a5/a9 for the training step: the same two kernels with the sample positions formed inside from the rays --
  * point (r, s) = rays_o[r] + rays_d[r] * t[r * t_ray_stride + s], multiply and add rounded separately exactly like
  * hbr_ray_points (vol_renderer.py:165, helper.py:48) -- so the (R*S,3) position tensor is never written or read.
