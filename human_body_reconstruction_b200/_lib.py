@@ -33,6 +33,7 @@ HBR_PEER_FLAG_BYTES = HBR_PEER_MAX_CTAS * HBR_MAX_PEERS * 4
 HBR_F32, HBR_F16, HBR_U8, HBR_BF16 = 0, 1, 2, 3
 HBR_ABI_VERSION = 2
 HBR_DFEAT_LEVEL_MAJOR = -1
+HBR_MC_BRICK, HBR_SCAN_TILE = 8, 4096
 
 
 class HashGeom(C.Structure):
@@ -217,6 +218,16 @@ SIGNATURES = {
     "hbr_mc_count": ([_vp, _i32, _i32, _i32, _f32, _i32, _i32, _vp, _vp], C.c_int),
     "hbr_mc_emit": ([_vp, _i32, _i32, _i32, _f32, _i32, _i32, _vp, _vp, _i64, _vp, _i64, _vp, _vp], C.c_int),
     "hbr_grid_interp": ([_vp, _i32, _i32, _i32, _i32, _vp, _i64, _vp, _vp], C.c_int),
+    "hbr_coarse_density": ([C.POINTER(C.c_double), C.POINTER(C.c_double), _i32, _vp, _geom_p, _vp, _dims_p, _vp, _vp, _vp, _i64,
+                            _i32, _vp], C.c_int),
+    "hbr_brick_density": ([C.POINTER(C.c_double), C.POINTER(C.c_double), _i32, _vp, _i64, _vp, _geom_p, _vp, _dims_p, _vp, _vp,
+                           _vp, _i64, _i32, _vp], C.c_int),
+    "hbr_brick_seed": ([_vp, _i32, _f32, _vp, _vp], C.c_int),
+    "hbr_brick_pending_count": ([_vp, _i32, _vp, _vp], C.c_int),
+    "hbr_brick_compact": ([_vp, _i32, _vp, _i32, _vp, _vp], C.c_int),
+    "hbr_brick_closure": ([_vp, _vp, _i64, _i32, _f32, _vp, _vp], C.c_int),
+    "hbr_brick_mc_count": ([_vp, _vp, _i64, _vp, _i32, _i32, _f32, _vp, _vp, _vp, _vp], C.c_int),
+    "hbr_brick_mc_emit": ([_vp, _vp, _i64, _vp, _i32, _i32, _f32, _vp, _vp, _vp, _vp, _vp], C.c_int),
 }
 
 # probes / self tests: a separate library (csrc/debug/ -> libhbr_b200_debug.so), not part of the product ABI
@@ -236,6 +247,8 @@ KERNELS_PER_CALL = {
     "hbr_composite_fwd": 1, "hbr_composite_bwd": 1, "hbr_composite_maps_fwd": 1, "hbr_composite_maps_bwd": 1, "hbr_strat_depths": 1, "hbr_mse_pair_fwd": 1, "hbr_mse_pair_bwd": 1, "hbr_mlp_tc_prepare": 1, "hbr_mlp_tc_reduce_grads": 1, "hbr_hier_sample": 1, "hbr_grid_points": 1,
     "hbr_composite_sdf_fwd": 1, "hbr_composite_sdf_bwd": 1, "hbr_sdf_stencil_points": 1, "hbr_sdf_eikonal_fwd": 1, "hbr_sdf_eikonal_bwd": 1,
     "hbr_grid_density": 3, "hbr_mlp_density_tf32x3": 1, "hbr_mc_count": 1, "hbr_mc_emit": 2, "hbr_grid_interp": 1,
+    "hbr_coarse_density": 3, "hbr_brick_density": 3, "hbr_brick_seed": 1, "hbr_brick_pending_count": 2, "hbr_brick_compact": 1,
+    "hbr_brick_closure": 1, "hbr_brick_mc_count": 7, "hbr_brick_mc_emit": 1,
 }
 
 

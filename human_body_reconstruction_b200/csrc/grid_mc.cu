@@ -16,18 +16,44 @@ __device__ __forceinline__ double linspace_at(double start, double stop, double 
   return __dadd_rn(__dmul_rn((double)i, step), start);      // arange(num)*step + start, no FMA
 }
 
+// grid point (i, j, k)  <->  (x[j], y[i], z[k])   (meshgrid default 'xy' indexing)
+__device__ __forceinline__ void grid_point(const GridAxes& ax, int i, int j, int k, __half* __restrict__ dst) {
+  dst[0] = __double2half(linspace_at(ax.start[0], ax.stop[0], ax.step[0], j, ax.res));
+  dst[1] = __double2half(linspace_at(ax.start[1], ax.stop[1], ax.step[1], i, ax.res));
+  dst[2] = __double2half(linspace_at(ax.start[2], ax.stop[2], ax.step[2], k, ax.res));
+}
+
 __global__ void grid_points_kernel(GridAxes ax, long long p0, long long count, __half* __restrict__ pts) {
   const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (q >= count) return;
   const long long p = p0 + q;
   const int res = ax.res;
-  const int k = (int)(p % res);
-  const int j = (int)((p / res) % res);
-  const int i = (int)(p / ((long long)res * res));
-  // flat index p = (i*res + j)*res + k  <->  (x[j], y[i], z[k])   (meshgrid default 'xy' indexing)
-  pts[q * 3 + 0] = __double2half(linspace_at(ax.start[0], ax.stop[0], ax.step[0], j, res));
-  pts[q * 3 + 1] = __double2half(linspace_at(ax.start[1], ax.stop[1], ax.step[1], i, res));
-  pts[q * 3 + 2] = __double2half(linspace_at(ax.start[2], ax.stop[2], ax.step[2], k, res));
+  // flat index p = (i*res + j)*res + k
+  grid_point(ax, (int)(p / ((long long)res * res)), (int)((p / res) % res), (int)(p % res), pts + q * 3);
+}
+
+// ---- the brick lattice of the sparse route (HBR_MC_BRICK^3 cells per brick, hbr.h) --------------------------------
+// coarse lattice point c = (ci*(nb+1) + cj)*(nb+1) + ck is grid point min(8c, res-1) per axis; points [q0, q0+count)
+__global__ void coarse_points_kernel(GridAxes ax, int nb, long long q0, long long count, __half* __restrict__ pts) {
+  const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= count) return;
+  const long long c = q0 + q;
+  const int m = nb + 1, last = ax.res - 1;
+  const int ci = (int)(c / ((long long)m * m)), cj = (int)((c / m) % m), ck = (int)(c % m);
+  grid_point(ax, min(ci * HBR_MC_BRICK, last), min(cj * HBR_MC_BRICK, last), min(ck * HBR_MC_BRICK, last), pts + q * 3);
+}
+
+// brick-major points: point q = s*729 + (li*9 + lj)*9 + lk is grid point min(8*B + l, res-1) per axis of brick B = bricks[s]
+__global__ void brick_points_kernel(GridAxes ax, int nb, const int32_t* __restrict__ bricks, long long q0, long long count,
+                                    __half* __restrict__ pts) {
+  constexpr int P = HBR_MC_BRICK + 1;
+  const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (q >= count) return;
+  const long long g = q0 + q;
+  const int b = __ldg(bricks + g / (P * P * P)), l = (int)(g % (P * P * P));
+  const int bi = b / (nb * nb), bj = (b / nb) % nb, bk = b % nb, last = ax.res - 1;
+  grid_point(ax, min(bi * HBR_MC_BRICK + l / (P * P), last), min(bj * HBR_MC_BRICK + (l / P) % P, last),
+             min(bk * HBR_MC_BRICK + l % P, last), pts + q * 3);
 }
 
 // ---- marching cubes ----------------------------------------------------------------------------------------
@@ -190,6 +216,17 @@ extern "C" int hbr_grid_interp(const float* vol, int C, int n0, int n1, int n2, 
   return HBR_OK;
 }
 
+static GridAxes make_axes(const double* min3, const double* max3, int res) {
+  GridAxes ax;
+  ax.res = res;
+  for (int a = 0; a < 3; ++a) {
+    ax.start[a] = min3[a];
+    ax.stop[a] = max3[a];
+    ax.step[a] = res > 1 ? (max3[a] - min3[a]) / (double)(res - 1) : 0.0;     // numpy: delta / div
+  }
+  return ax;
+}
+
 extern "C" int hbr_grid_points(const double* min3, const double* max3, int res, int64_t p0, int64_t count,
                                void* pts_f16, void* stream) {
   HBR_REQUIRE(min3 && max3 && res >= 1, "bad argument");
@@ -198,22 +235,18 @@ extern "C" int hbr_grid_points(const double* min3, const double* max3, int res, 
               (long long)p0, (long long)count, res);
   if (count == 0) return HBR_OK;
   HBR_REQUIRE(pts_f16 != nullptr, "NULL pointer");
-  GridAxes ax;
-  ax.res = res;
-  for (int a = 0; a < 3; ++a) {
-    ax.start[a] = min3[a];
-    ax.stop[a] = max3[a];
-    ax.step[a] = res > 1 ? (max3[a] - min3[a]) / (double)(res - 1) : 0.0;     // numpy: delta / div
-  }
-  grid_points_kernel<<<(unsigned)ceil_div(count, 256), 256, 0, as_stream(stream)>>>(ax, p0, count, (__half*)pts_f16);
+  grid_points_kernel<<<(unsigned)ceil_div(count, 256), 256, 0, as_stream(stream)>>>(make_axes(min3, max3, res), p0, count,
+                                                                                   (__half*)pts_f16);
   HBR_LAUNCH_CHECK();
   return HBR_OK;
 }
 
-extern "C" int hbr_grid_density(const double* min3, const double* max3, int res, int64_t p0, int64_t count,
-                                const float* table, const hbr_hash_geom* geom, const float* params,
-                                const hbr_mlp_dims* dims, const float* dir_enc, float* out, void* pts_scratch,
-                                float* feat_scratch, int64_t chunk, int field_mode, void* stream) {
+// The field at `count` points whose fp16 positions points(s, c) writes to pts_scratch for points [s, s+c), chunk by chunk:
+// encoder -> density head (or the full MLP with dir_enc).  Every dense and sparse density query runs through here.
+template <class Points>
+static int field_at_points(Points&& points, int64_t count, const float* table, const hbr_hash_geom* geom,
+                           const float* params, const hbr_mlp_dims* dims, const float* dir_enc, float* out,
+                           void* pts_scratch, float* feat_scratch, int64_t chunk, int field_mode, void* stream) {
   HBR_REQUIRE(geom && dims && chunk >= 1, "bad argument");
   HBR_REQUIRE(field_mode == 0 || field_mode == 1, "field_mode %d", field_mode);
   HBR_REQUIRE(dims->in0 == geom->L * geom->F + geom->E, "MLP input width %d != encoder width %d", dims->in0,
@@ -221,7 +254,7 @@ extern "C" int hbr_grid_density(const double* min3, const double* max3, int res,
   const int ow = dir_enc ? 4 : 1;
   for (int64_t s = 0; s < count; s += chunk) {
     const int64_t c = count - s < chunk ? count - s : chunk;
-    if (int rc = hbr_grid_points(min3, max3, res, p0 + s, c, pts_scratch, stream)) return rc;
+    if (int rc = points(s, c)) return rc;
     if (int rc = hbr_hash_encode_fwd(pts_scratch, HBR_F16, c, table, geom, feat_scratch, dims->in0, stream)) return rc;
     if (!dir_enc && field_mode == 0 && dims->in0 == 32) {
       if (int rc = hbr_mlp_density_tf32x3(feat_scratch, c, params, dims, out + s, stream)) return rc;
@@ -232,6 +265,52 @@ extern "C" int hbr_grid_density(const double* min3, const double* max3, int res,
       return rc;
   }
   return HBR_OK;
+}
+
+extern "C" int hbr_grid_density(const double* min3, const double* max3, int res, int64_t p0, int64_t count,
+                                const float* table, const hbr_hash_geom* geom, const float* params,
+                                const hbr_mlp_dims* dims, const float* dir_enc, float* out, void* pts_scratch,
+                                float* feat_scratch, int64_t chunk, int field_mode, void* stream) {
+  return field_at_points([&](int64_t s, int64_t c) { return hbr_grid_points(min3, max3, res, p0 + s, c, pts_scratch, stream); },
+                         count, table, geom, params, dims, dir_enc, out, pts_scratch, feat_scratch, chunk, field_mode, stream);
+}
+
+static int brick_count(int res) { return res >= 2 ? (int)ceil_div(res - 1, HBR_MC_BRICK) : 0; }
+
+extern "C" int hbr_coarse_density(const double* min3, const double* max3, int res, const float* table,
+                                  const hbr_hash_geom* geom, const float* params, const hbr_mlp_dims* dims, float* out,
+                                  void* pts_scratch, float* feat_scratch, int64_t chunk, int field_mode, void* stream) {
+  HBR_REQUIRE(min3 && max3 && res >= 2, "bad argument (res %d < 2)", res);
+  HBR_REQUIRE(out && pts_scratch && feat_scratch, "NULL pointer");
+  const int nb = brick_count(res);
+  const int64_t count = (int64_t)(nb + 1) * (nb + 1) * (nb + 1);
+  const GridAxes ax = make_axes(min3, max3, res);
+  auto points = [&](int64_t s, int64_t c) {
+    coarse_points_kernel<<<(unsigned)ceil_div(c, 256), 256, 0, as_stream(stream)>>>(ax, nb, s, c, (__half*)pts_scratch);
+    HBR_LAUNCH_CHECK();
+    return (int)HBR_OK;
+  };
+  return field_at_points(points, count, table, geom, params, dims, nullptr, out, pts_scratch, feat_scratch, chunk, field_mode,
+                         stream);
+}
+
+extern "C" int hbr_brick_density(const double* min3, const double* max3, int res, const int32_t* bricks, int64_t n,
+                                 const float* table, const hbr_hash_geom* geom, const float* params,
+                                 const hbr_mlp_dims* dims, float* out, void* pts_scratch, float* feat_scratch, int64_t chunk,
+                                 int field_mode, void* stream) {
+  HBR_REQUIRE(min3 && max3 && res >= 2 && n >= 0, "bad argument");
+  if (n == 0) return HBR_OK;
+  HBR_REQUIRE(bricks && out && pts_scratch && feat_scratch, "NULL pointer");
+  const int nb = brick_count(res);
+  constexpr int P = HBR_MC_BRICK + 1;
+  const GridAxes ax = make_axes(min3, max3, res);
+  auto points = [&](int64_t s, int64_t c) {
+    brick_points_kernel<<<(unsigned)ceil_div(c, 256), 256, 0, as_stream(stream)>>>(ax, nb, bricks, s, c, (__half*)pts_scratch);
+    HBR_LAUNCH_CHECK();
+    return (int)HBR_OK;
+  };
+  return field_at_points(points, n * P * P * P, table, geom, params, dims, nullptr, out, pts_scratch, feat_scratch, chunk,
+                         field_mode, stream);
 }
 
 static int check_mc(const float* d, int n0, int n1, int n2, int i_begin, int i_end) {

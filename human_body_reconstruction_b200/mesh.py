@@ -16,6 +16,7 @@ import torch
 import torch.nn as nn
 
 from . import ops
+from ._lib import HBR_MC_BRICK
 from .encoder import PositionalEncoder
 from .hash_encoding import HashEncoder
 from .test_hash import MLP_3D
@@ -197,11 +198,84 @@ def index_to_world(verts: torch.Tensor, axes: torch.Tensor) -> torch.Tensor:
     return torch.stack((w[1], w[0], w[2]), dim=1).contiguous()
 
 
+# ---------------------------------------------------------------------------------------------------------------
+# sparse marching cubes: the same res^3 grid, evaluated and meshed only in the 8^3-cell bricks the surface passes through
+# ---------------------------------------------------------------------------------------------------------------
+class SparseSurface(NamedTuple):
+    """vertices (V,3) fp32 grid-index coordinates and faces (F,3) int32 in marching_cubes' conventions; bricks (n,) int32:
+    the active bricks in slot order (closure round by round, brick-index order within a round); rounds: field
+    evaluations of brick lists (seeds included); points: field values used ((nb+1)^3 coarse + 729 per active brick)."""
+    vertices: torch.Tensor
+    faces: torch.Tensor
+    bricks: torch.Tensor
+    rounds: int
+    points: int
+
+
+def select_bricks(coarse: torch.Tensor, iso: float, brick_density):
+    """Seed and close the active brick set.  coarse: the (nb+1)^3 coarse-lattice values; brick_density(bricks) -> (n,9,9,9)
+    values of the listed bricks.  Seeds are the bricks whose 8 corner values straddle iso; each round evaluates the bricks
+    activated by the last one and activates the face neighbours across every interior 9x9 boundary plane that straddles
+    iso, until no brick is added.  Returns (brick map (nb,nb,nb) int32: slot or -1, bricks in slot order, their values
+    (n,9,9,9), rounds)."""
+    bmap = ops.brick_seed(coarse, iso)
+    lists, dens, rounds, base = [], [], 0, 0
+    while True:
+        lst = ops.brick_compact(bmap, base)
+        if lst.shape[0] == 0:
+            break
+        d = brick_density(lst)
+        ops.brick_closure(d, lst, bmap, iso)
+        lists.append(lst)
+        dens.append(d)
+        base += lst.shape[0]
+        rounds += 1
+    P = HBR_MC_BRICK + 1
+    if not lists:
+        return bmap, torch.empty((0,), device=bmap.device, dtype=torch.int32), \
+            torch.empty((0, P, P, P), device=bmap.device, dtype=torch.float32), 0
+    return bmap, torch.cat(lists), torch.cat(dens), rounds
+
+
+def sparse_surface_index(res: int, iso: float, coarse: torch.Tensor, brick_density) -> SparseSurface:
+    """Sparse marching cubes of the res^3 grid whose values at the coarse lattice are `coarse` and on bricks
+    `brick_density(bricks)` gives (select_bricks): seed, closure rounds, then one welded vertex per crossing edge of the
+    active bricks' cells.  The result equals marching_cubes of the dense grid restricted to those cells; it is the dense
+    mesh when every crossing cell lies in an active brick.  A surface component that crosses no coarse-lattice edge of a
+    brick and never reaches a seeded brick through crossing boundary planes is not meshed.  Vertex and face order is a
+    deterministic function of the brick list."""
+    if res < 2:
+        raise ValueError(f"res {res} < 2")
+    if tuple(coarse.shape) != (ops.brick_count(res) + 1,) * 3:
+        raise ValueError(f"coarse lattice {tuple(coarse.shape)} does not match res {res}")
+    bmap, bricks, dens, rounds = select_bricks(coarse, iso, brick_density)
+    verts, faces = ops.brick_mc(dens, bricks, bmap, res, iso)
+    return SparseSurface(verts, faces, bricks, rounds, coarse.numel() + dens.numel())
+
+
+def sparse_field_surface(encoder: HashEncoder, nerf, min_bound, max_bound, res: int, iso: float, chunk: int = 1 << 19,
+                         cuda_core_mlp: bool = False) -> SparseSurface:
+    """sparse_surface_index on the field: coarse lattice and bricks evaluated with density_grid's positions, encoder and
+    density head, so every value equals density_grid's at the same grid index."""
+    table, geom, params, dims = _native_field(encoder, nerf)
+    mn, mx = [float(v) for v in min_bound], [float(v) for v in max_bound]
+    with torch.no_grad():
+        coarse = ops.coarse_density(mn, mx, res, table, geom, params, dims, chunk, cuda_core_mlp)
+        return sparse_surface_index(res, iso, coarse, lambda b: ops.brick_density(mn, mx, res, b, table, geom, params, dims,
+                                                                                  chunk, cuda_core_mlp))
+
+
 def extract_mesh(encoder: HashEncoder, nerf, dir_encoder: PositionalEncoder, min_bound, max_bound, res: int = 256,
-                 iso: float = 30.0, chunk: int = 1 << 20) -> Mesh:
+                 iso: float = 30.0, chunk: int = 1 << 20, sparse: bool = False) -> Mesh:
     """Checkpoint -> oriented, coloured, world-space mesh: density_grid (density only, the tensor-core path) ->
     world_surface (marching_cubes, index_to_world, winding) -> normals and colours at the world vertices
     (vertex_attributes).
+
+    sparse=True replaces density_grid + marching_cubes by sparse_field_surface: the same grid, evaluated and meshed only in
+    the 8^3-cell bricks reached from the coarse lattice's crossings (memory and time follow the surface, not res^3).  It
+    gives the dense mesh whenever every crossing cell lies in an active brick, and drops a component that fits inside one
+    brick without crossing a coarse-lattice edge and never touches a seeded brick.  Its vertex and face order is
+    deterministic.
 
     Conventions:
     * World mapping: index axis 0 is y, 1 is x, 2 is z; each axis maps through fp16(linspace(min, max, res)), the
@@ -212,9 +286,21 @@ def extract_mesh(encoder: HashEncoder, nerf, dir_encoder: PositionalEncoder, min
     * Colours: the field's raw RGB (ELU output, not clamped) seen head-on, view direction -n ((0,0,1) where n = 0).
     * Order: vertex and face order follow hbr_mc_emit's atomic cursors and are NOT stable across runs; every per-vertex
       value is a deterministic function of the vertex position."""
+    if sparse:
+        surf = sparse_field_surface(encoder, nerf, min_bound, max_bound, res, iso)
+        return index_surface_mesh(encoder, nerf, dir_encoder, surf.vertices, surf.faces, min_bound, max_bound, res, chunk)
     dens = density_grid(encoder, nerf, None, min_bound, max_bound, res)
     verts, faces = world_surface(dens, iso, min_bound, max_bound)
     del dens
+    normals, colors = vertex_attributes(encoder, nerf, dir_encoder, verts, chunk)
+    return Mesh(verts, faces, normals, colors)
+
+
+def index_surface_mesh(encoder: HashEncoder, nerf, dir_encoder: PositionalEncoder, vidx: torch.Tensor, faces: torch.Tensor,
+                       min_bound, max_bound, res: int, chunk: int = 1 << 20) -> Mesh:
+    """extract_mesh's steps after marching cubes, for a surface in grid-index coordinates of the res^3 grid (marching_cubes'
+    or sparse_surface_index's conventions): index_to_world, the winding swap, normals and colours."""
+    verts, faces = _index_to_world_surface(vidx, faces, min_bound, max_bound, res)
     normals, colors = vertex_attributes(encoder, nerf, dir_encoder, verts, chunk)
     return Mesh(verts, faces, normals, colors)
 
@@ -228,6 +314,10 @@ def world_surface(density: torch.Tensor, iso: float, min_bound, max_bound) -> Tu
     if tuple(density.shape) != (res, res, res):
         raise ValueError(f"expected a (res,res,res) grid, got {tuple(density.shape)}")
     vidx, faces = marching_cubes(density, iso)
+    return _index_to_world_surface(vidx, faces, min_bound, max_bound, res)
+
+
+def _index_to_world_surface(vidx, faces, min_bound, max_bound, res):
     verts = index_to_world(vidx, world_axes(min_bound, max_bound, res, vidx.device))
     return verts, faces[:, [0, 2, 1]].contiguous()
 

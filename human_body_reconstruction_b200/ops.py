@@ -910,6 +910,97 @@ def mc_emit(density: torch.Tensor, iso: float, n_verts: int, n_faces: int):
     return verts[:n_verts], faces[:n_faces], cursors
 
 
+def brick_count(res: int) -> int:
+    """nb: bricks per axis of the sparse route's lattice over a res^3 grid (hbr.h, sparse marching cubes)."""
+    return -(-(res - 1) // _lib.HBR_MC_BRICK)
+
+
+def _field_density(fn, n_points, min_bound, max_bound, res, table, geom, params, dims, lead, chunk, cuda_core_mlp):
+    require_cuda(table, params)
+    mn = (C.c_double * 3)(*[float(v) for v in min_bound])
+    mx = (C.c_double * 3)(*[float(v) for v in max_bound])
+    chunk = max(1, min(chunk, n_points))
+    dev = table.device
+    out = torch.empty((n_points,), device=dev, dtype=torch.float32)
+    pts = torch.empty((chunk, 3), device=dev, dtype=torch.float16)
+    feat = torch.empty((chunk, dims.in0), device=dev, dtype=torch.float32)
+    check(fn(mn, mx, res, *lead, ptr(table), C.byref(geom), ptr(params), C.byref(dims), ptr(out), ptr(pts), ptr(feat), chunk,
+             1 if cuda_core_mlp else 0, stream()))
+    return out
+
+
+def coarse_density(min_bound, max_bound, res, table, geom, params, dims, chunk=1 << 19, cuda_core_mlp=False) -> torch.Tensor:
+    """Density at the coarse lattice: (nb+1)^3 fp32, the grid points min(8c, res-1) per axis (grid_density's values)."""
+    m = brick_count(res) + 1
+    return _field_density(lib().hbr_coarse_density, m ** 3, min_bound, max_bound, res, table, geom, params, dims, (), chunk,
+                          cuda_core_mlp).view(m, m, m)
+
+
+def brick_density(min_bound, max_bound, res, bricks, table, geom, params, dims, chunk=1 << 19, cuda_core_mlp=False) -> torch.Tensor:
+    """Density on the 9^3 points of each listed brick (int32 brick indices): (n, 9, 9, 9) fp32, indices clamped to res-1."""
+    require_cuda(bricks)
+    bricks = bricks.to(torch.int32).contiguous()
+    n = bricks.shape[0]
+    P = _lib.HBR_MC_BRICK + 1
+    if n == 0:
+        return torch.empty((0, P, P, P), device=bricks.device, dtype=torch.float32)
+    return _field_density(lib().hbr_brick_density, n * P ** 3, min_bound, max_bound, res, table, geom, params, dims,
+                          (ptr(bricks), n), chunk, cuda_core_mlp).view(n, P, P, P)
+
+
+def brick_seed(coarse: torch.Tensor, iso: float) -> torch.Tensor:
+    """Brick map (nb,nb,nb) int32 from the coarse lattice (nb+1)^3: HBR_BRICK_PENDING (-2) where a brick's 8 corner values
+    straddle iso, HBR_BRICK_INACTIVE (-1) elsewhere."""
+    require_cuda(coarse)
+    coarse = _f32c(coarse)
+    nb = coarse.shape[0] - 1
+    bmap = torch.empty((nb, nb, nb), device=coarse.device, dtype=torch.int32)
+    check(lib().hbr_brick_seed(ptr(coarse), nb, float(iso), ptr(bmap), stream()))
+    return bmap
+
+
+def brick_compact(bmap: torch.Tensor, base: int) -> torch.Tensor:
+    """The pending bricks of bmap in brick-index order (int32); they get the slots base, base+1, ... in bmap.  One host read
+    (the count)."""
+    require_cuda(bmap)
+    nb = bmap.shape[0]
+    sums = torch.empty((-(-nb ** 3 // _lib.HBR_SCAN_TILE) + 1,), device=bmap.device, dtype=torch.int64)
+    check(lib().hbr_brick_pending_count(ptr(bmap), nb, ptr(sums), stream()))
+    n = int(sums[-1])
+    lst = torch.empty((n,), device=bmap.device, dtype=torch.int32)
+    if n:
+        check(lib().hbr_brick_compact(ptr(bmap), nb, ptr(sums), base, ptr(lst), stream()))
+    return lst
+
+
+def brick_closure(dens: torch.Tensor, bricks: torch.Tensor, bmap: torch.Tensor, iso: float) -> None:
+    """Marks PENDING the inactive face neighbours of the listed bricks whose shared 9x9 plane straddles iso (in place)."""
+    require_cuda(dens, bricks, bmap)
+    dens = _f32c(dens)
+    check(lib().hbr_brick_closure(ptr(dens), ptr(bricks), bricks.shape[0], bmap.shape[0], float(iso), ptr(bmap), stream()))
+
+
+def brick_mc(dens: torch.Tensor, bricks: torch.Tensor, bmap: torch.Tensor, res: int, iso: float):
+    """Marching cubes over the cells of the bricks in slot order (bricks[s] in slot s, dens (n,9,9,9)): (verts (V,3) fp32 in
+    grid-index coordinates, faces (F,3) int32), welded across bricks.  One host read (the totals)."""
+    require_cuda(dens, bricks, bmap)
+    dens, bricks = _f32c(dens), bricks.to(torch.int32).contiguous()
+    n, nb, dev = bricks.shape[0], bmap.shape[0], bmap.device
+    P = _lib.HBR_MC_BRICK + 1
+    eid = torch.empty((n, 3, P, P, P), device=dev, dtype=torch.uint16)
+    offsets = torch.empty((n + 1, 2), device=dev, dtype=torch.int64)
+    sums = torch.empty((-(-n // _lib.HBR_SCAN_TILE) + 1,), device=dev, dtype=torch.int64)
+    check(lib().hbr_brick_mc_count(ptr(dens), ptr(bricks), n, ptr(bmap), nb, res, float(iso), ptr(eid), ptr(offsets), ptr(sums),
+                                   stream()))
+    nv, nt = offsets[n].tolist()
+    verts = torch.empty((nv, 3), device=dev, dtype=torch.float32)
+    faces = torch.empty((nt, 3), device=dev, dtype=torch.int32)
+    if nv or nt:
+        check(lib().hbr_brick_mc_emit(ptr(dens), ptr(bricks), n, ptr(bmap), nb, res, float(iso), ptr(eid), ptr(offsets),
+                                      ptr(verts), ptr(faces), stream()))
+    return verts, faces
+
+
 def grid_interp(vol: torch.Tensor, pts: torch.Tensor) -> torch.Tensor:
     """vol (C,n0,n1,n2) fp32, pts (n,3) as (x,y,z) = (axis 2, axis 1, axis 0) index coordinates -> (n,C)."""
     require_cuda(vol, pts)

@@ -375,6 +375,51 @@ int hbr_mc_emit(const float* density, int n0, int n1, int n2, float iso, int i_b
                 int32_t* edge_id, float* verts, int64_t max_verts, int32_t* faces, int64_t max_faces,
                 unsigned long long* cursors, void* stream);
 
+/* ---- sparse marching cubes: the res^3 grid above, meshed brick by brick ---------------------------------------------
+ * A brick is HBR_MC_BRICK^3 cells; nb = ceil((res-1)/8) bricks per axis, brick b = (bi*nb + bj)*nb + bk holds the cells
+ * [8B, min(8B+8, res-1)) per axis and is evaluated on its 9^3 points, indices past res-1 clamped to res-1.  Brick
+ * densities are brick-major (n, 9, 9, 9) fp32.  The coarse lattice is the (nb+1)^3 grid points min(8c, res-1), flat index
+ * (ci*(nb+1) + cj)*(nb+1) + ck.  Positions are hbr_grid_points' fp16 values and the field is hbr_grid_density's (same
+ * field_mode, dir_enc = NULL), so every value equals the dense grid's at the same index.
+ * The brick map (nb^3 int32) holds HBR_BRICK_INACTIVE, HBR_BRICK_PENDING (to be evaluated) or the brick's slot >= 0: its
+ * row in the caller's brick-density and scratch arrays.  Scans run in tiles of HBR_SCAN_TILE entries; `block_sums` is
+ * ceil(n / HBR_SCAN_TILE) + 1 int64. */
+#define HBR_MC_BRICK 8
+#define HBR_BRICK_INACTIVE (-1)
+#define HBR_BRICK_PENDING (-2)
+#define HBR_SCAN_TILE 4096
+/* pts_scratch: (chunk,3) halfs, feat_scratch: (chunk, L*F+E) floats.  out: (nb+1)^3 floats. */
+int hbr_coarse_density(const double* min3_host, const double* max3_host, int res, const float* table,
+                       const hbr_hash_geom* geom_host, const float* params, const hbr_mlp_dims* dims, float* out,
+                       void* pts_scratch, float* feat_scratch, int64_t chunk, int field_mode, void* stream);
+/* out: (n, 9, 9, 9) floats for the bricks listed in bricks (n int32 brick indices). */
+int hbr_brick_density(const double* min3_host, const double* max3_host, int res, const int32_t* bricks, int64_t n,
+                      const float* table, const hbr_hash_geom* geom_host, const float* params, const hbr_mlp_dims* dims,
+                      float* out, void* pts_scratch, float* feat_scratch, int64_t chunk, int field_mode, void* stream);
+/* Seed: map[b] = PENDING where the 8 coarse values at brick b's corners are not all on one side of iso, else INACTIVE. */
+int hbr_brick_seed(const float* coarse, int nb, float iso, int32_t* map, void* stream);
+/* Compaction of the PENDING bricks in brick-index order, by a scan (no atomics).  hbr_brick_pending_count writes the
+ * per-tile counts, exclusively scanned, to block_sums and the total to block_sums[ceil(nb^3 / HBR_SCAN_TILE)];
+ * hbr_brick_compact then writes list[m] = the m-th pending brick and sets its map entry to the slot base + m. */
+int hbr_brick_pending_count(const int32_t* map, int nb, int64_t* block_sums, void* stream);
+int hbr_brick_compact(int32_t* map, int nb, const int64_t* block_sums, int32_t base, int32_t* list, void* stream);
+/* Closure step over the n bricks just evaluated (list, their densities dens (n,9,9,9)): each of a brick's 6 boundary
+ * planes of 9x9 points that is not on the outer grid boundary and holds points on both sides of iso makes the neighbour
+ * across it PENDING if it was INACTIVE. */
+int hbr_brick_closure(const float* dens, const int32_t* list, int64_t n, int nb, float iso, int32_t* map, void* stream);
+/* Marching cubes over the cells of the n bricks in slot order (list[s] = the brick in slot s, dens (n,9,9,9)); every map
+ * entry is INACTIVE or a slot.  A crossing grid edge gets one vertex, emitted by the first active brick among those
+ * containing it, in the order o, o-e_u, o-e_v, o-e_u-e_v (o = min(p/8, nb-1) of its lower end point p; u < v the other
+ * axes, a step back only where p lies on an interior brick plane).
+ * hbr_brick_mc_count writes the local vertex id of every (point, axis) of each brick to eid (n, 3, 9, 9, 9) uint16
+ * (0xffff: no vertex of this brick) and offsets (n+1, 2) int64: the exclusive scans of the per-brick vertex and triangle
+ * counts, totals in row n.  hbr_brick_mc_emit writes vertices (grid-index coordinates along axes 0,1,2, the dense
+ * route's arithmetic) and triangles (the dense route's tables and winding): brick s's go to the rows from offsets[s]. */
+int hbr_brick_mc_count(const float* dens, const int32_t* list, int64_t n, const int32_t* map, int nb, int res, float iso,
+                       uint16_t* eid, int64_t* offsets, int64_t* block_sums, void* stream);
+int hbr_brick_mc_emit(const float* dens, const int32_t* list, int64_t n, const int32_t* map, int nb, int res, float iso,
+                      const uint16_t* eid, const int64_t* offsets, float* verts, int32_t* faces, void* stream);
+
 /* a14: torchmcubes.grid_interp (nerf2mesh.py:99): trilinear samples of vol (C, n0, n1, n2) fp32 at pts (n,3) given as
  * (x, y, z) = (index along axis 2, axis 1, axis 0) in grid-index units (the order torchmcubes returns vertices in),
  * clamped to the volume; out (n, C). */

@@ -5,10 +5,13 @@ nerf2mesh.py:56-65): HashEncoder(N_min=16, N_max=max_res, L=16, F=2, T=2**hash_s
 sigma=|max_bound - min_bound|_2), PositionalEncoder(3, 4), MLP_3D(num_sig=2, num_col=2, L=16, F=2, d_view=24).  The
 checkpoint loads through formats.load_checkpoint (with or without nn.DataParallel's `module.` prefix); the mesh comes
 from mesh.extract_mesh and is written by mesh.write_ply (vertex x y z nx ny nz red green blue, faces counter-clockwise
-seen from outside).
+seen from outside).  With --sparse the grid is evaluated and meshed only in the 8^3-cell bricks the surface passes through
+(mesh.sparse_field_surface): memory and time follow the surface, so the field's finest resolution (--res 2048) fits; a
+component that crosses no brick corner edge and never reaches a seeded brick is not meshed.  The JSON line then also
+reports the active bricks and closure rounds.
 
 usage: python scripts/export_mesh.py --ckpt_name NAME --bound_pth bounds_model.npy --hash_size 19
-                                     [--max_res 2048] [--res 256] [--iso 30.0] [--out mesh.ply]
+                                     [--max_res 2048] [--res 256] [--iso 30.0] [--sparse] [--out mesh.ply]
 """
 from __future__ import annotations
 
@@ -48,19 +51,27 @@ def main(argv=None):
     ap.add_argument("--max_res", type=float, default=2048.0, help="N_max of the hash encoder the field was trained with")
     ap.add_argument("--res", type=int, default=256, help="density-grid resolution per axis")
     ap.add_argument("--iso", type=float, default=30.0, help="density iso level of the surface")
+    ap.add_argument("--sparse", action="store_true", help="mesh only the 8^3-cell bricks the surface passes through")
     ap.add_argument("--out", default="mesh.ply", help="output PLY path")
     args = ap.parse_args(argv)
     if not torch.cuda.is_available():
         raise SystemExit("export_mesh.py needs a CUDA device")
     enc, nerf, dir_enc, mn, mx = build_field(args.ckpt_name, args.bound_pth, args.hash_size, args.max_res)
     t0 = time.perf_counter()
-    m = mesh.extract_mesh(enc, nerf, dir_enc, mn, mx, res=args.res, iso=args.iso)
+    extra = {}
+    if args.sparse:
+        surf = mesh.sparse_field_surface(enc, nerf, mn, mx, args.res, args.iso)
+        extra = {"active_bricks": int(surf.bricks.shape[0]), "rounds": surf.rounds}
+        m = mesh.index_surface_mesh(enc, nerf, dir_enc, surf.vertices, surf.faces, mn, mx, args.res)
+        del surf
+    else:
+        m = mesh.extract_mesh(enc, nerf, dir_enc, mn, mx, res=args.res, iso=args.iso)
     torch.cuda.synchronize()
     t1 = time.perf_counter()
     mesh.write_ply(args.out, m)
     t2 = time.perf_counter()
     print(json.dumps({"out": args.out, "vertices": int(m.vertices.shape[0]), "faces": int(m.faces.shape[0]),
-                      "extract_s": t1 - t0, "write_s": t2 - t1}))
+                      "extract_s": t1 - t0, "write_s": t2 - t1, **extra}))
 
 
 if __name__ == "__main__":
