@@ -228,6 +228,7 @@ SIGNATURES = {
     "hbr_brick_closure": ([_vp, _vp, _i64, _i32, _f32, _vp, _vp], C.c_int),
     "hbr_brick_mc_count": ([_vp, _vp, _i64, _vp, _i32, _i32, _f32, _vp, _vp, _vp, _vp], C.c_int),
     "hbr_brick_mc_emit": ([_vp, _vp, _i64, _vp, _i32, _i32, _f32, _vp, _vp, _vp, _vp, _vp], C.c_int),
+    "hbr_mesh_components": ([_vp, _i64, _i64, _vp, _vp, _vp, _vp], C.c_int),
 }
 
 # probes / self tests: a separate library (csrc/debug/ -> libhbr_b200_debug.so), not part of the product ABI
@@ -248,7 +249,7 @@ KERNELS_PER_CALL = {
     "hbr_composite_sdf_fwd": 1, "hbr_composite_sdf_bwd": 1, "hbr_sdf_stencil_points": 1, "hbr_sdf_eikonal_fwd": 1, "hbr_sdf_eikonal_bwd": 1,
     "hbr_grid_density": 3, "hbr_mlp_density_tf32x3": 1, "hbr_mc_count": 1, "hbr_mc_emit": 2, "hbr_grid_interp": 1,
     "hbr_coarse_density": 3, "hbr_brick_density": 3, "hbr_brick_seed": 1, "hbr_brick_pending_count": 2, "hbr_brick_compact": 1,
-    "hbr_brick_closure": 1, "hbr_brick_mc_count": 7, "hbr_brick_mc_emit": 1,
+    "hbr_brick_closure": 1, "hbr_brick_mc_count": 7, "hbr_brick_mc_emit": 1, "hbr_mesh_components": 4,
 }
 
 

@@ -265,10 +265,74 @@ def sparse_field_surface(encoder: HashEncoder, nerf, min_bound, max_bound, res: 
                                                                                   chunk, cuda_core_mlp))
 
 
+# ---------------------------------------------------------------------------------------------------------------
+# floaters: connected components of a mesh, and keeping the ones that matter
+# ---------------------------------------------------------------------------------------------------------------
+class MeshComponents(NamedTuple):
+    """labels (V,) int32: the smallest vertex index of each vertex's component; roots (C,) int64: the components' root
+    indices (labels[r] == r), ascending; faces / vertices (C,) int64: each component's face and vertex count, in roots'
+    order (a face belongs to the component of its first vertex)."""
+    labels: torch.Tensor
+    roots: torch.Tensor
+    faces: torch.Tensor
+    vertices: torch.Tensor
+
+
+def mesh_components(faces: torch.Tensor, nv: int) -> MeshComponents:
+    """Connected components of the mesh whose (F,3) faces index nv vertices (hbr_mesh_components on the GPU): two vertices
+    are connected when a chain of faces joins them; a vertex no face uses is a component of its own."""
+    labels, face_count, vertex_count = ops.mesh_components(faces, nv)
+    roots = torch.nonzero(vertex_count).squeeze(1)             # every root counts itself; every other index holds 0
+    return MeshComponents(labels, roots, face_count[roots].long(), vertex_count[roots].long())
+
+
+def keep_components(comp: MeshComponents, min_faces: int = 0, largest: Optional[int] = None) -> torch.Tensor:
+    """bool (C,): the components with >= min_faces faces that are, when largest = k is given, also among the k largest by
+    face count.  Every component tied with the k-th largest count is kept, so the choice depends on the mesh as a set, not
+    on its vertex order.  The defaults keep everything."""
+    keep = comp.faces >= min_faces
+    if largest is not None:
+        if largest < 1:
+            raise ValueError(f"largest = {largest}: keep at least one component (or pass None)")
+        if largest < comp.faces.shape[0]:
+            keep &= comp.faces >= torch.topk(comp.faces, largest).values[-1]
+    return keep
+
+
+def filter_surface(vertices: torch.Tensor, faces: torch.Tensor, keep_vertex: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Stable compaction of a mesh to the vertices where keep_vertex (V,) bool holds and the faces whose three vertices are
+    all kept: (vertex_index (V',) int64 -- the kept vertices' rows of `vertices`, ascending -- and the kept faces (F',3)
+    int32 re-indexed to them, in their original order)."""
+    if tuple(keep_vertex.shape) != (vertices.shape[0],) or keep_vertex.dtype != torch.bool:
+        raise ValueError(f"keep_vertex must be ({vertices.shape[0]},) bool, got {tuple(keep_vertex.shape)} {keep_vertex.dtype}")
+    faces = faces.to(torch.int32)
+    new_id = torch.cumsum(keep_vertex, 0, dtype=torch.int32) - 1            # V <= 2^31 - 1 (hbr_mesh_components)
+    kept = faces[keep_vertex.index_select(0, faces.reshape(-1)).view(-1, 3).all(1)]
+    return torch.nonzero(keep_vertex).squeeze(1), new_id.index_select(0, kept.reshape(-1)).view(-1, 3)
+
+
+def filter_by_components(vertices: torch.Tensor, faces: torch.Tensor, min_faces: int = 0, largest: Optional[int] = None):
+    """mesh_components -> keep_components -> filter_surface: (vertex_index, faces', the components, their keep mask)."""
+    comp = mesh_components(faces, vertices.shape[0])
+    keep = keep_components(comp, min_faces, largest)
+    keep_root = torch.zeros((vertices.shape[0],), device=faces.device, dtype=torch.bool)
+    keep_root[comp.roots[keep]] = True
+    vertex_index, faces = filter_surface(vertices, faces, keep_root.index_select(0, comp.labels))
+    return vertex_index, faces, comp, keep
+
+
+def filter_components(m: Mesh, min_faces: int = 0, largest: Optional[int] = None) -> Mesh:
+    """The mesh without its floaters: the components keep_components keeps, compacted stably (filter_surface).  Positions,
+    normals and colours of the kept vertices are gathered, so each stays bitwise what it was."""
+    vi, faces, _, _ = filter_by_components(m.vertices, m.faces, min_faces, largest)
+    return Mesh(m.vertices[vi], faces, m.normals[vi], m.colors[vi])
+
+
 def extract_mesh(encoder: HashEncoder, nerf, dir_encoder: PositionalEncoder, min_bound, max_bound, res: int = 256,
-                 iso: float = 30.0, chunk: int = 1 << 20, sparse: bool = False) -> Mesh:
+                 iso: float = 30.0, chunk: int = 1 << 20, sparse: bool = False, min_component_faces: int = 0,
+                 largest_components: Optional[int] = None) -> Mesh:
     """Checkpoint -> oriented, coloured, world-space mesh: density_grid (density only, the tensor-core path) ->
-    world_surface (marching_cubes, index_to_world, winding) -> normals and colours at the world vertices
+    marching_cubes -> index_to_world and the winding swap -> normals and colours at the world vertices
     (vertex_attributes).
 
     sparse=True replaces density_grid + marching_cubes by sparse_field_surface: the same grid, evaluated and meshed only in
@@ -276,6 +340,10 @@ def extract_mesh(encoder: HashEncoder, nerf, dir_encoder: PositionalEncoder, min
     gives the dense mesh whenever every crossing cell lies in an active brick, and drops a component that fits inside one
     brick without crossing a coarse-lattice edge and never touches a seeded brick.  Its vertex and face order is
     deterministic.
+
+    min_component_faces / largest_components drop floaters (keep_components' rule) right after marching cubes, in grid-index
+    space, so no attribute work is spent on them; the result equals filter_components of the unfiltered mesh.  With the
+    defaults no labelling runs.
 
     Conventions:
     * World mapping: index axis 0 is y, 1 is x, 2 is z; each axis maps through fp16(linspace(min, max, res)), the
@@ -287,13 +355,15 @@ def extract_mesh(encoder: HashEncoder, nerf, dir_encoder: PositionalEncoder, min
     * Order: vertex and face order follow hbr_mc_emit's atomic cursors and are NOT stable across runs; every per-vertex
       value is a deterministic function of the vertex position."""
     if sparse:
-        surf = sparse_field_surface(encoder, nerf, min_bound, max_bound, res, iso)
-        return index_surface_mesh(encoder, nerf, dir_encoder, surf.vertices, surf.faces, min_bound, max_bound, res, chunk)
-    dens = density_grid(encoder, nerf, None, min_bound, max_bound, res)
-    verts, faces = world_surface(dens, iso, min_bound, max_bound)
-    del dens
-    normals, colors = vertex_attributes(encoder, nerf, dir_encoder, verts, chunk)
-    return Mesh(verts, faces, normals, colors)
+        vidx, faces = sparse_field_surface(encoder, nerf, min_bound, max_bound, res, iso)[:2]
+    else:
+        dens = density_grid(encoder, nerf, None, min_bound, max_bound, res)
+        vidx, faces = marching_cubes(dens, iso)
+        del dens
+    if min_component_faces > 0 or largest_components is not None:
+        vi, faces, _, _ = filter_by_components(vidx, faces, min_component_faces, largest_components)
+        vidx = vidx[vi]
+    return index_surface_mesh(encoder, nerf, dir_encoder, vidx, faces, min_bound, max_bound, res, chunk)
 
 
 def index_surface_mesh(encoder: HashEncoder, nerf, dir_encoder: PositionalEncoder, vidx: torch.Tensor, faces: torch.Tensor,

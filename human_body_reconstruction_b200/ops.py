@@ -1001,6 +1001,28 @@ def brick_mc(dens: torch.Tensor, bricks: torch.Tensor, bmap: torch.Tensor, res: 
     return verts, faces
 
 
+def mesh_components(faces: torch.Tensor, nv: int):
+    """Connected components of the mesh whose (F,3) integer faces index nv vertices (hbr_mesh_components): (label,
+    face_count, vertex_count), int32 (nv,) each.  label[v] is the smallest vertex index of v's component; the sizes sit at
+    the roots (label[r] == r) and are 0 elsewhere.  Every index must lie in [0, nv) (ValueError otherwise, checked by one
+    reduction before anything is launched)."""
+    if faces.dim() != 2 or faces.shape[1] != 3 or faces.dtype.is_floating_point or faces.dtype.is_complex or \
+            faces.dtype == torch.bool:
+        raise ValueError(f"faces must be an (F,3) integer tensor, got {tuple(faces.shape)} {faces.dtype}")
+    nv = int(nv)
+    if not 0 <= nv <= 0x7fffffff:
+        raise ValueError(f"nv {nv} outside [0, 2^31 - 1]")
+    if faces.shape[0]:
+        lo, hi = (int(x) for x in torch.aminmax(faces))
+        if lo < 0 or hi >= nv:
+            raise ValueError(f"face indices span [{lo}, {hi}], outside [0, {nv})")
+    require_cuda(faces)
+    faces = faces.to(torch.int32).contiguous()
+    label, face_count, vertex_count = (torch.empty((nv,), device=faces.device, dtype=torch.int32) for _ in range(3))
+    check(lib().hbr_mesh_components(ptr(faces), faces.shape[0], nv, ptr(label), ptr(face_count), ptr(vertex_count), stream()))
+    return label, face_count, vertex_count
+
+
 def grid_interp(vol: torch.Tensor, pts: torch.Tensor) -> torch.Tensor:
     """vol (C,n0,n1,n2) fp32, pts (n,3) as (x,y,z) = (axis 2, axis 1, axis 0) index coordinates -> (n,C)."""
     require_cuda(vol, pts)

@@ -420,6 +420,15 @@ int hbr_brick_mc_count(const float* dens, const int32_t* list, int64_t n, const 
 int hbr_brick_mc_emit(const float* dens, const int32_t* list, int64_t n, const int32_t* map, int nb, int res, float iso,
                       const uint16_t* eid, const int64_t* offsets, float* verts, int32_t* faces, void* stream);
 
+/* ---- connected components of a triangle mesh (floater removal after marching cubes) -------------------------------
+ * faces (nf, 3) int32 index nv vertices (0 <= nv <= INT32_MAX; indices are NOT range-checked here).  Two vertices are
+ * connected when a chain of faces joins them through shared vertices; a vertex no face uses is its own component.
+ * label[v] = the smallest vertex index of v's component; face_count[r] / vertex_count[r] = the component's faces (a face
+ * belongs to the component of its first vertex) and vertices at its root r (label[r] == r), 0 at every other index.  All
+ * three nv-int32 outputs are written in full; the result does not depend on thread order. */
+int hbr_mesh_components(const int32_t* faces, int64_t nf, int64_t nv, int32_t* label, int32_t* face_count,
+                        int32_t* vertex_count, void* stream);
+
 /* a14: torchmcubes.grid_interp (nerf2mesh.py:99): trilinear samples of vol (C, n0, n1, n2) fp32 at pts (n,3) given as
  * (x, y, z) = (index along axis 2, axis 1, axis 0) in grid-index units (the order torchmcubes returns vertices in),
  * clamped to the volume; out (n, C). */

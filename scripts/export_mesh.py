@@ -8,10 +8,13 @@ from mesh.extract_mesh and is written by mesh.write_ply (vertex x y z nx ny nz r
 seen from outside).  With --sparse the grid is evaluated and meshed only in the 8^3-cell bricks the surface passes through
 (mesh.sparse_field_surface): memory and time follow the surface, so the field's finest resolution (--res 2048) fits; a
 component that crosses no brick corner edge and never reaches a seeded brick is not meshed.  The JSON line then also
-reports the active bricks and closure rounds.
+reports the active bricks and closure rounds.  --min-component-faces N / --largest-components K drop floaters (mesh
+components with fewer than N faces / outside the K largest by face count, ties kept: mesh.keep_components) before the
+normals and colours are computed; the JSON line then also reports the components before filtering and those kept.
 
 usage: python scripts/export_mesh.py --ckpt_name NAME --bound_pth bounds_model.npy --hash_size 19
-                                     [--max_res 2048] [--res 256] [--iso 30.0] [--sparse] [--out mesh.ply]
+                                     [--max_res 2048] [--res 256] [--iso 30.0] [--sparse] [--min-component-faces N]
+                                     [--largest-components K] [--out mesh.ply]
 """
 from __future__ import annotations
 
@@ -52,6 +55,9 @@ def main(argv=None):
     ap.add_argument("--res", type=int, default=256, help="density-grid resolution per axis")
     ap.add_argument("--iso", type=float, default=30.0, help="density iso level of the surface")
     ap.add_argument("--sparse", action="store_true", help="mesh only the 8^3-cell bricks the surface passes through")
+    ap.add_argument("--min-component-faces", type=int, default=0, help="drop mesh components with fewer faces")
+    ap.add_argument("--largest-components", type=int, default=None,
+                    help="keep only the K largest components by face count (ties with the K-th kept)")
     ap.add_argument("--out", default="mesh.ply", help="output PLY path")
     args = ap.parse_args(argv)
     if not torch.cuda.is_available():
@@ -59,13 +65,21 @@ def main(argv=None):
     enc, nerf, dir_enc, mn, mx = build_field(args.ckpt_name, args.bound_pth, args.hash_size, args.max_res)
     t0 = time.perf_counter()
     extra = {}
+    # extract_mesh's steps, spelled out for the counts the JSON line reports
     if args.sparse:
         surf = mesh.sparse_field_surface(enc, nerf, mn, mx, args.res, args.iso)
         extra = {"active_bricks": int(surf.bricks.shape[0]), "rounds": surf.rounds}
-        m = mesh.index_surface_mesh(enc, nerf, dir_enc, surf.vertices, surf.faces, mn, mx, args.res)
+        vidx, faces = surf.vertices, surf.faces
         del surf
     else:
-        m = mesh.extract_mesh(enc, nerf, dir_enc, mn, mx, res=args.res, iso=args.iso)
+        dens = mesh.density_grid(enc, nerf, None, mn, mx, args.res)
+        vidx, faces = mesh.marching_cubes(dens, args.iso)
+        del dens
+    if args.min_component_faces > 0 or args.largest_components is not None:
+        vi, faces, comp, kept = mesh.filter_by_components(vidx, faces, args.min_component_faces, args.largest_components)
+        vidx = vidx[vi]
+        extra.update(components=int(comp.roots.shape[0]), components_kept=int(kept.sum()))
+    m = mesh.index_surface_mesh(enc, nerf, dir_enc, vidx, faces, mn, mx, args.res)
     torch.cuda.synchronize()
     t1 = time.perf_counter()
     mesh.write_ply(args.out, m)
