@@ -13,7 +13,8 @@ twice); the last backward node of a module publishes its buffer (the encoder in 
 scatter-add kernel has been enqueued) and the exchange of a published piece may start right there, overlapping what is
 left of the backward; an end-of-backward engine callback reduces the rest, makes the compute stream wait, and only then
 hands the buffers to `.grad`.  MSE is a mean over the LOCAL batch, so the average over ranks equals the single-process
-gradient of the concatenated batch.
+gradient of the concatenated batch.  The modules' side of this protocol -- what every autograd node of HashEncoder /
+MLP_3D does with or without an exchange attached -- is `node_params` and `ParamGrad`, below `_GradExchange`.
 """
 from __future__ import annotations
 
@@ -214,6 +215,95 @@ class _GradExchange:
             for k in self._fwd:
                 self._fwd[k] = 0
                 self._pub[k] = []
+
+
+def node_params(*modules) -> list:
+    """The parameters an autograd node of these modules is applied with.  Under no_grad they are passed detached: the node
+    decides from needs_input_grad, which follows requires_grad and not the grad mode, whether to count itself with the
+    exchange or pre-zero a table gradient buffer, and no backward would ever read either."""
+    ps = [p for m in modules for p in m._dp_params()]
+    return ps if torch.is_grad_enabled() else [p.detach() for p in ps]
+
+
+class ParamGrad:
+    """One autograd node's gradient of one module's parameters (HashEncoder tables or MLP_3D), created in the node's
+    forward and kept on ctx.  `wanted`: whether the node's parameter inputs need a gradient.  When they do, the forward
+    notes the node with the module's exchange or, without one, starts the module's side-stream pre-zero
+    (HashEncoder._zeroed_grad_async).  In the backward:
+
+        buffer()            the flat buffer to accumulate into: the exchange's, the pre-zeroed one or fresh zeros
+        stream_plan(n)      the level chunks of a streamed exchange (only the last table node under one), else None
+        scatter_table(...)  the table's scatter-add schedule: one level range, level chunks or a streamed exchange
+        complete(piece)     a finished piece (default: the whole buffer); the last node under an exchange publishes it
+        grads()             what the node returns to autograd for the parameters; ends the node's backward"""
+
+    def __init__(self, m, wanted: bool):
+        self.m, self.wanted = m, bool(wanted)
+        self.exchange = m._dp if wanted else None
+        self.buf, self.last, self._pre = None, False, None
+        self._flat = m._flat                  # the storage the forward ran with (its _flat_table() / _flat_params())
+        if self.exchange is not None:
+            self.exchange.note_forward(m)
+        elif wanted and hasattr(type(m), "_zeroed_grad_async"):
+            self._pre = m._zeroed_grad_async()
+
+    def buffer(self) -> torch.Tensor:
+        if self.buf is None:
+            if self.exchange is not None:
+                self.buf, self.last = self.exchange.enter_backward(self.m)
+            elif self._pre is not None:
+                self.buf, ev = self._pre
+                self._pre = None
+                torch.cuda.current_stream().wait_event(ev)
+            else:
+                self.buf = torch.zeros_like(self._flat)
+        return self.buf
+
+    def stream_plan(self, n_points: int):
+        if self.exchange is None:
+            return None
+        self.buffer()
+        return self.exchange.stream_plan(self.m, self.m.L, n_points) if self.last else None
+
+    def complete(self, piece: torch.Tensor | None = None):
+        if self.exchange is not None and self.last:
+            self.exchange.publish(self.m, self.buf if piece is None else piece)
+
+    def grads(self) -> tuple:
+        buf, self.buf, self.last = self.buf, None, False          # a retained graph's next backward starts afresh
+        if self.exchange is not None or not self.wanted:
+            return (None,) * len(self.m._dp_params())             # the exchange hands its buffer to .grad
+        return tuple(self.m._grad_views(buf))
+
+    def scatter_table(self, run, n_points: int, stream=None, after_first=None, mlp: "ParamGrad | None" = None,
+                      mlp_stream=None):
+        """Enqueues the table gradient.  run(g, l0, l1): the scatter-add of levels [l0, l1) into g.  One level range,
+        except in the last node under an exchange: level chunks, each published as soon as its scatter-add is enqueued,
+        so its all-reduce overlaps the next chunk's scatter-add.  With `stream` and a streamed exchange (stream_plan):
+        stream(g, chunks, done) enqueues ONE scatter-add launch that finishes the chunks in order and returns the count a
+        chunk's done word reaches, and the exchange is ONE launch beside it on the exchange's side stream.  That launch
+        also carries the gradient of `mlp` when it is the same exchange's last MLP node, once `mlp_stream` (the stream
+        finishing it, or None) gets there.  after_first() runs behind the first chunk's scatter-add, or behind the
+        streamed exchange's launch."""
+        g = self.buffer()
+        plan = self.stream_plan(n_points) if stream is not None else None
+        if plan is not None:
+            ev_pre = torch.cuda.current_stream().record_event()
+            need = stream(g, plan, self.exchange.done)
+            with_mlp = mlp is not None and mlp.exchange is self.exchange and mlp.last
+            ev_mlp = mlp_stream.record_event() if (mlp_stream is not None and with_mlp) else None
+            self.exchange.exchange_streamed(plan, need, after=(ev_pre, ev_mlp), include_mlp=with_mlp)
+            if with_mlp:
+                mlp.last = False                                  # published by that launch
+            if after_first is not None:
+                after_first()
+            return
+        L = self.m.L
+        for l0, l1 in (self.exchange.level_chunks(self.m, L, n_points) if self.last else [(0, L)]):
+            run(g, l0, l1)
+            if l0 == 0 and after_first is not None:
+                after_first()
+            self.complete(g[l0:l1])
 
 
 class GradAllReduce(_GradExchange):

@@ -14,6 +14,7 @@ import torch.nn as nn
 from torch.autograd.function import once_differentiable
 
 from . import ops
+from .dist import ParamGrad, node_params
 
 
 class _HashEncodeFn(torch.autograd.Function):
@@ -26,55 +27,27 @@ class _HashEncodeFn(torch.autograd.Function):
         ctx.geom = geom
         ctx.table = table if ctx.needs_input_grad[0] else None     # the tables the positions' gradient is taken at
         ctx.save_for_backward(x)
-        ctx.g = None
-        if any(ctx.needs_input_grad[2:]):
-            if enc._dp is not None:
-                enc._dp.note_forward(enc)
-            else:
-                ctx.g = enc._zeroed_grad_async()
+        ctx.grad = ParamGrad(enc, any(ctx.needs_input_grad[2:]))
         return y
 
     @staticmethod
     @once_differentiable
     def backward(ctx, dy):
         (x,) = ctx.saved_tensors
-        enc = ctx.enc
-        L, T, F = enc.L, enc.T, enc.F
-        dp = enc._dp
         # HashEncoder.position_grad: dL/dx through the trilinear weights (first order only)
         dx = ops.hash_encode_dx(x, ctx.table, ctx.geom, dy).to(x.dtype) if ctx.table is not None else None
         ctx.table = None
-        if not any(ctx.needs_input_grad[2:]):       # positions only (frozen tables): no table gradient to form
-            return (dx, None) + (None,) * L
-        if dp is not None:
-            # Data-parallel run (dist._GradExchange): accumulate into the persistent buffer of this backward pass.  The
-            # last table backward of the pass runs in level chunks and publishes each one as soon as its scatter-add is
-            # enqueued: that chunk's all-reduce travels over NVLink while the next chunk's scatter-add still runs.  The
-            # exchange hands the reduced buffer to .grad at the end of backward; nothing is returned to autograd here.
-            g, last = dp.enter_backward(enc)
-            plan = dp.stream_plan(enc, L, x.shape[0]) if last else None
-            if plan is not None:
-                # streamed exchange (dist.PeerGradAllReduce(streamed=True)): one scatter-add launch finishing the level
-                # chunks in order, one exchange launch beside it on the reducer's side stream
-                ev_pre = torch.cuda.current_stream().record_event()
-                ops.hash_encode_bwd_stream(x, dy[:, : L * F], ctx.geom, g, plan, dp.done)
-                dp.exchange_streamed(plan, ops.hash_bwd_stream_tiles(x.shape[0]), after=(ev_pre,))
-                return (dx, None) + (None,) * L
-            for l0, l1 in (dp.level_chunks(enc, L, x.shape[0]) if last else [(0, L)]):
-                ops.hash_encode_bwd(x, dy[:, : L * F], ctx.geom, g, l0, l1)
-                if last:
-                    dp.publish(enc, g[l0:l1])
-            return (dx, None) + (None,) * L
-        if ctx.g is not None:
-            g, ev = ctx.g
-            ctx.g = None
-            torch.cuda.current_stream().wait_event(ev)
-        else:
-            g = torch.zeros((L, T, F), device=dy.device, dtype=torch.float32)
-        ops.hash_encode_bwd(x, dy[:, : L * F], ctx.geom, g, 0, L)
+        if ctx.grad.wanted:                         # frozen tables: positions only, no table gradient to form
+            dy = dy[:, : ctx.enc.L * ctx.enc.F]
+
+            def stream(g, chunks, done):
+                ops.hash_encode_bwd_stream(x, dy, ctx.geom, g, chunks, done)
+                return ops.hash_bwd_stream_tiles(x.shape[0])
+
+            ctx.grad.scatter_table(lambda g, l0, l1: ops.hash_encode_bwd(x, dy, ctx.geom, g, l0, l1), x.shape[0], stream)
         # no gradient w.r.t. x unless position_grad is set: the reference detaches the interpolation weights
         # (hash_encoding.py:160)
-        return (dx, None) + tuple(g[i] for i in range(L))
+        return (dx, None) + ctx.grad.grads()
 
 
 class HashEncoder(nn.Module):
@@ -176,11 +149,17 @@ class HashEncoder(nn.Module):
         return g, ev
 
     # -- data-parallel gradient exchange (dist._GradExchange) ---------------------------------------------------
+    def _dp_params(self):
+        return [e.weight for e in self.Embedding_list]
+
     def _dp_template(self) -> torch.Tensor:
         return self._flat_table()
 
+    def _grad_views(self, buf: torch.Tensor):
+        return [buf[i] for i in range(self.L)]
+
     def _dp_param_views(self, buf: torch.Tensor):
-        return [(e.weight, buf[i]) for i, e in enumerate(self.Embedding_list)]
+        return list(zip(self._dp_params(), self._grad_views(buf)))
 
     def level_scales(self):
         return list(self._scales)
@@ -202,10 +181,5 @@ class HashEncoder(nn.Module):
         table = self._flat_table()
         if table.device != x.device:
             raise RuntimeError(f"encoder tables are on {table.device}, x on {x.device}")
-        weights = [e.weight for e in self.Embedding_list]
-        if not torch.is_grad_enabled():
-            # needs_input_grad follows requires_grad, not the grad mode: under no_grad the node would still zero a table
-            # gradient buffer that no backward ever reads
-            weights = [w.detach() for w in weights]
         keep = getattr(self, "position_grad", False) and x.requires_grad and torch.is_grad_enabled()
-        return _HashEncodeFn.apply(x if keep else x.detach(), self, *weights)
+        return _HashEncodeFn.apply(x if keep else x.detach(), self, *node_params(self))

@@ -18,6 +18,7 @@ import torch.nn as nn
 
 from . import ops
 from ._lib import MlpDims
+from .dist import ParamGrad, node_params
 
 
 class _MlpFn(torch.autograd.Function):
@@ -34,8 +35,7 @@ class _MlpFn(torch.autograd.Function):
             out, act = ops.mlp_fwd_tc(feat, dirs, dir_group, flat, dims, keep_act=train, operand=use_tc)
         else:
             out, act = ops.mlp_fwd_f32(feat, dirs, dir_group, flat, dims, keep_act=train)
-        if mlp._dp is not None and any(ctx.needs_input_grad[5:]):
-            mlp._dp.note_forward(mlp)
+        ctx.grad = ParamGrad(mlp, any(ctx.needs_input_grad[5:]))
         ctx.mlp, ctx.dims, ctx.dir_group, ctx.use_tc = mlp, dims, dir_group, use_tc
         ctx.save_for_backward(feat, dirs, out if use_tc else act)     # the tensor-core backward reads the saved output
         return out
@@ -45,11 +45,7 @@ class _MlpFn(torch.autograd.Function):
         feat, dirs, act = ctx.saved_tensors
         mlp = ctx.mlp
         flat = mlp._flat_params()
-        dp = mlp._dp if any(ctx.needs_input_grad[5:]) else None
-        if dp is not None:
-            dflat, last = dp.enter_backward(mlp)      # persistent buffer of this backward pass, accumulated into
-        else:
-            dflat, last = torch.zeros_like(flat), False
+        dflat = ctx.grad.buffer()
         dout = dout.float().contiguous()
         want_dfeat, want_ddirs = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
         if ctx.use_tc:
@@ -57,11 +53,8 @@ class _MlpFn(torch.autograd.Function):
                                           dflat, operand=ctx.use_tc, grad_scale=mlp.tc_grad_scale)
         else:
             dfeat, ddirs = ops.mlp_bwd_f32(feat, dirs, ctx.dir_group, flat, ctx.dims, dout, act, want_dfeat, want_ddirs, dflat)
-        if dp is not None:
-            if last:
-                dp.publish(mlp, dflat)
-            return (dfeat, ddirs, None, None, None) + (None,) * len(mlp._ordered())
-        return (dfeat, ddirs, None, None, None) + tuple(mlp._grad_views(dflat))
+        ctx.grad.complete()
+        return (dfeat, ddirs, None, None, None) + ctx.grad.grads()
 
 
 class _DensityFn(torch.autograd.Function):
@@ -76,8 +69,7 @@ class _DensityFn(torch.autograd.Function):
         train = any(ctx.needs_input_grad)
         feat = feat.float().contiguous()
         out, act = ops.mlp_fwd_f32(feat, None, 1, flat, dims, keep_act=train)
-        if mlp._dp is not None and any(ctx.needs_input_grad[2:]):
-            mlp._dp.note_forward(mlp)
+        ctx.grad = ParamGrad(mlp, any(ctx.needs_input_grad[2:]))
         ctx.mlp, ctx.dims = mlp, dims
         ctx.save_for_backward(feat, act)
         return out
@@ -85,19 +77,12 @@ class _DensityFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dout):
         feat, act = ctx.saved_tensors
-        mlp = ctx.mlp
-        flat = mlp._flat_params()
-        dp = mlp._dp if any(ctx.needs_input_grad[2:]) else None
-        if dp is not None:
-            dflat, last = dp.enter_backward(mlp)
-        else:
-            dflat, last = torch.zeros_like(flat), False
-        dfeat, _ = ops.mlp_bwd_f32(feat, None, 1, flat, ctx.dims, dout.float().contiguous(), act, ctx.needs_input_grad[0], False, dflat)
-        if dp is not None:
-            if last:
-                dp.publish(mlp, dflat)
-            return (dfeat, None) + (None,) * len(mlp._ordered())
-        return (dfeat, None) + tuple(mlp._grad_views(dflat))
+        flat = ctx.mlp._flat_params()
+        dflat = ctx.grad.buffer()
+        dfeat, _ = ops.mlp_bwd_f32(feat, None, 1, flat, ctx.dims, dout.float().contiguous(), act, ctx.needs_input_grad[0], False,
+                                   dflat)
+        ctx.grad.complete()
+        return (dfeat, None) + ctx.grad.grads()
 
 
 class MLP_3D(nn.Module):
@@ -193,6 +178,8 @@ class MLP_3D(nn.Module):
     def _dims(self) -> MlpDims:
         return MlpDims(self._in0, self.d_view)
 
+    _dp_params = _ordered
+
     def _dp_template(self) -> torch.Tensor:
         return self._flat_params()
 
@@ -218,7 +205,7 @@ class MLP_3D(nn.Module):
         """(N,4) [rgb, density].  With use_sdf the density column is 2*sigmoid(pre-activation) - 1 (test_hash.py:59-60)
         unless raw=True."""
         self._check_native()
-        out = _MlpFn.apply(feat, dirs_enc, int(dir_group), self, self._tc_operand(use_tc), *self._ordered())
+        out = _MlpFn.apply(feat, dirs_enc, int(dir_group), self, self._tc_operand(use_tc), *node_params(self))
         if self.use_sdf and not raw:
             out = torch.cat((out[:, :3], self._sdf_from_density(out[:, 3:4])), dim=-1)
         return out
@@ -239,7 +226,7 @@ class MLP_3D(nn.Module):
                 z = torch.zeros((x.shape[0], self.d_view), device=x.device)
                 return self.field(x, z, 1, use_tc=None, raw=True)[:, 3:4]       # 16-bit tensor-core kernels (whole field)
             self._check_native()
-            return _DensityFn.apply(x, self, *self._ordered())
+            return _DensityFn.apply(x, self, *node_params(self))
         density, _ = ops.mlp_fwd_f32(x.float().contiguous(), None, 1, self._flat_params(), self._dims(), keep_act=False)
         return density
 

@@ -19,6 +19,7 @@ import torch
 import torch.nn as nn
 
 from . import ops
+from .dist import ParamGrad, node_params
 from .encoder import PositionalEncoder
 from .hash_encoding import HashEncoder
 from .helper import calc_color, hierarchical_sampling, strat_sampler
@@ -36,35 +37,22 @@ class _FieldFn(torch.autograd.Function):
         operand = ops.tc_operand()
         out, feat16 = ops.field_fwd_tc(pts, enc._flat_table(), geom, dirs, dir_group, mlp._flat_params(), dims, operand)
         ctx.enc, ctx.mlp, ctx.geom, ctx.dims, ctx.dir_group, ctx.operand = enc, mlp, geom, dims, dir_group, operand
-        if enc._dp is not None:
-            enc._dp.note_forward(enc)
-            mlp._dp.note_forward(mlp)
+        ctx.tab_grad = ParamGrad(enc, any(ctx.needs_input_grad[5:5 + enc.L]))
+        ctx.mlp_grad = ParamGrad(mlp, any(ctx.needs_input_grad[5 + enc.L:]))
         ctx.save_for_backward(pts, dirs, feat16, out)
         return out
 
     @staticmethod
     def backward(ctx, dout):
         pts, dirs, feat16, out = ctx.saved_tensors
-        enc, mlp = ctx.enc, ctx.mlp
-        L, T, F = enc.L, enc.T, enc.F
-        flat = mlp._flat_params()
-        dp = enc._dp
-        if dp is not None:
-            g, last_e = dp.enter_backward(enc)
-            dflat, last_m = mlp._dp.enter_backward(mlp)
-        else:
-            g = torch.zeros((L, T, F), device=dout.device, dtype=torch.float32)
-            dflat = torch.zeros_like(flat)
-        ddirs = ops.field_bwd_tc(pts, ctx.geom, dirs, ctx.dir_group, flat, ctx.dims, feat16, out.detach(),
+        tab, mlp = ctx.tab_grad, ctx.mlp_grad
+        g, dflat = tab.buffer(), mlp.buffer()
+        ddirs = ops.field_bwd_tc(pts, ctx.geom, dirs, ctx.dir_group, ctx.mlp._flat_params(), ctx.dims, feat16, out.detach(),
                                  dout.float().contiguous(), g, ctx.needs_input_grad[1], dflat, operand=ctx.operand,
-                                 grad_scale=mlp.tc_grad_scale)
-        if dp is not None:
-            if last_m:
-                mlp._dp.publish(mlp, dflat)
-            if last_e:
-                dp.publish(enc, g)
-            return (None, ddirs, None, None, None) + (None,) * (L + len(mlp._ordered()))
-        return (None, ddirs, None, None, None) + tuple(g[i] for i in range(L)) + tuple(mlp._grad_views(dflat))
+                                 grad_scale=ctx.mlp.tc_grad_scale)
+        mlp.complete()
+        tab.complete()
+        return (None, ddirs, None, None, None) + tab.grads() + mlp.grads()
 
 
 class _FieldRaysFn(torch.autograd.Function):
@@ -101,114 +89,66 @@ class _FieldRaysFn(torch.autograd.Function):
             out, _ = ops.mlp_fwd_tc(feat16, dirs, S, flat, dims, operand=operand, image_ready=True)
         ctx.enc, ctx.mlp, ctx.geom, ctx.dims, ctx.S, ctx.operand = enc, mlp, geom, dims, S, operand
         ctx.save_for_backward(rays_o, rays_d, t, dirs, feat16, out)
-        ctx.want_tab = any(ctx.needs_input_grad[6:6 + enc.L])
-        ctx.want_mlp = any(ctx.needs_input_grad[6 + enc.L:])
-        ctx.g = None
-        if ctx.want_tab:
-            if enc._dp is not None:
-                enc._dp.note_forward(enc)
-            else:
-                ctx.g = enc._zeroed_grad_async()
-        if ctx.want_mlp and mlp._dp is not None:
-            mlp._dp.note_forward(mlp)
+        ctx.tab_grad = ParamGrad(enc, any(ctx.needs_input_grad[6:6 + enc.L]))
+        ctx.mlp_grad = ParamGrad(mlp, any(ctx.needs_input_grad[6 + enc.L:]))
         return out
 
     @staticmethod
     def backward(ctx, dout):
         rays_o, rays_d, t, dirs, feat16, out = ctx.saved_tensors
-        enc, mlp = ctx.enc, ctx.mlp
-        L, T, F = enc.L, enc.T, enc.F
-        flat = mlp._flat_params()
-        dpm = mlp._dp if ctx.want_mlp else None
-        if dpm is not None:
-            dflat, last_m = dpm.enter_backward(mlp)
-        else:
-            dflat, last_m = torch.zeros_like(flat), False
+        tab, mlp = ctx.tab_grad, ctx.mlp_grad
+        flat = ctx.mlp._flat_params()
+        dflat = mlp.buffer()
+        n_pts = feat16.shape[0]
         # single GPU, the reference's configuration family: ONE kernel -- the scatter-add into the table gradient runs on
         # dedicated warps of the MLP backward kernel, tile by tile (hbr_field_bwd_rays_tc); the gradient exchange of the
         # multi-GPU path publishes level chunks of the table gradient while the scatter-add is still running, so it keeps
         # the two-kernel form below
         # (measured: 0.467 against 0.477 ms per 4 096-ray step; at 131 072 rays the two kernels, each at full occupancy,
         # are 1 % ahead, hence the size limit)
-        if (FUSE_SCATTER and ctx.want_tab and ctx.want_mlp and enc._dp is None and dpm is None
-                and feat16.shape[0] <= FUSE_SCATTER_MAX_POINTS and ops.field_scatter_supported(ctx.geom, ctx.dims)):
-            if ctx.g is not None:
-                g, ev = ctx.g
-                ctx.g = None
-                torch.cuda.current_stream().wait_event(ev)
-            else:
-                g = torch.zeros((L, T, F), device=dout.device, dtype=torch.float32)
+        if (FUSE_SCATTER and tab.wanted and mlp.wanted and tab.exchange is None and mlp.exchange is None
+                and n_pts <= FUSE_SCATTER_MAX_POINTS and ops.field_scatter_supported(ctx.geom, ctx.dims)):
+            g = tab.buffer()
             ddirs = ops.field_bwd_rays_tc(feat16, rays_o, rays_d, t, ctx.geom, dirs, flat, ctx.dims, out.detach(),
                                           dout.float().contiguous(), g, ctx.needs_input_grad[3], dflat, operand=ctx.operand,
-                                          grad_scale=mlp.tc_grad_scale, defer_reduce=False)
-            return (None, None, None, ddirs, None, None) + tuple(g[i] for i in range(L)) + tuple(mlp._grad_views(dflat))
+                                          grad_scale=ctx.mlp.tc_grad_scale, defer_reduce=False)
+            return (None, None, None, ddirs, None, None) + tab.grads() + mlp.grads()
         # the reduction of the MLP kernel's per-CTA gradient rows runs on a side stream, beside the hash-grid backward
-        defer = ctx.want_tab
-        n_pts = feat16.shape[0]
-        dpe = enc._dp if ctx.want_tab else None
-        plan, lm = None, False
-        if dpe is not None:
-            g, last = dpe.enter_backward(enc)
-            # streamed exchange (dist.PeerGradAllReduce(streamed=True)): the last table backward of the pass finishes the
-            # table gradient level chunk by level chunk while the all-reduce kernel beside it sends the finished chunks; the
-            # MLP kernel then writes d(features) level-major for the level-major scatter-add
-            plan = dpe.stream_plan(enc, L, n_pts) if last else None
-            lm = plan is not None and STREAM_LEVEL_MAJOR and ops.mlp_level_major_ok(ctx.geom, ctx.dims, n_pts)
-        dfeat, ddirs = ops.mlp_bwd_tc(feat16, dirs, ctx.S, flat, ctx.dims, out.detach(), dout.float().contiguous(), ctx.want_tab,
-                                      ctx.needs_input_grad[3], dflat, operand=ctx.operand, grad_scale=mlp.tc_grad_scale,
+        defer = tab.wanted
+        # streamed exchange (dist.PeerGradAllReduce(streamed=True)): the last table backward of the pass finishes the table
+        # gradient level chunk by level chunk while the all-reduce kernel beside it sends the finished chunks; the MLP kernel
+        # then writes d(features) level-major for the level-major scatter-add
+        plan = tab.stream_plan(n_pts)
+        lm = plan is not None and STREAM_LEVEL_MAJOR and ops.mlp_level_major_ok(ctx.geom, ctx.dims, n_pts)
+        dfeat, ddirs = ops.mlp_bwd_tc(feat16, dirs, ctx.S, flat, ctx.dims, out.detach(), dout.float().contiguous(), tab.wanted,
+                                      ctx.needs_input_grad[3], dflat, operand=ctx.operand, grad_scale=ctx.mlp.tc_grad_scale,
                                       defer_reduce=defer, level_major=lm)
         cur, side = torch.cuda.current_stream(), _side_stream(dout.device)
         if defer:
             side.wait_stream(cur)
             with torch.cuda.stream(side):
-                ops.mlp_tc_reduce_grads(ctx.dims, feat16.shape[0], dflat, dout.device)
+                ops.mlp_tc_reduce_grads(ctx.dims, n_pts, dflat, dout.device)
             dflat.record_stream(side)
 
         def join_mlp():
             if defer:
                 cur.wait_stream(side)
-            if dpm is not None and last_m:
-                dpm.publish(mlp, dflat)
+            mlp.complete()
 
-        gm = (None,) * len(mlp._ordered()) if (dpm is not None or not ctx.want_mlp) else tuple(mlp._grad_views(dflat))
-        if not ctx.want_tab:
-            join_mlp()
-            return (None, None, None, ddirs, None, None) + (None,) * L + gm
-        if dpe is not None:
-            if plan is not None:
-                # ONE scatter-add launch that finishes the level chunks in order, ONE exchange launch on the reducer's side
-                # stream beside it (it waits for the MLP kernels only, not for the scatter-add)
-                ev_pre = cur.record_event()
-                if lm:
-                    ops.hash_encode_bwd_rays_lm(rays_o, rays_d, t, dfeat, ctx.geom, g, plan, dpe.done)
-                    need = ops.hash_bwd_lm_ctas(n_pts)
-                else:
-                    ops.hash_encode_bwd_rays_stream(rays_o, rays_d, t, dfeat, ctx.geom, g, plan, dpe.done)
-                    need = ops.hash_bwd_stream_tiles(n_pts)
-                with_mlp = dpm is dpe and last_m
-                ev_mlp = side.record_event() if (defer and with_mlp) else None
-                dpe.exchange_streamed(plan, need, after=(ev_pre, ev_mlp), include_mlp=with_mlp)
-                if defer:
-                    cur.wait_stream(side)
-                if dpm is not None and last_m and not with_mlp:
-                    dpm.publish(mlp, dflat)
-                return (None, None, None, ddirs, None, None) + (None,) * L + gm
-            for l0, l1 in (dpe.level_chunks(enc, L, feat16.shape[0]) if last else [(0, L)]):
-                ops.hash_encode_bwd_rays(rays_o, rays_d, t, dfeat, ctx.geom, g, l0, l1)
-                if l0 == 0:
-                    join_mlp()                      # the MLP gradient is complete (and published) behind the first chunk
-                if last:
-                    dpe.publish(enc, g[l0:l1])
-            return (None, None, None, ddirs, None, None) + (None,) * L + gm
-        if ctx.g is not None:
-            g, ev = ctx.g
-            ctx.g = None
-            torch.cuda.current_stream().wait_event(ev)
+        def stream(g, chunks, done):
+            if lm:
+                ops.hash_encode_bwd_rays_lm(rays_o, rays_d, t, dfeat, ctx.geom, g, chunks, done)
+                return ops.hash_bwd_lm_ctas(n_pts)
+            ops.hash_encode_bwd_rays_stream(rays_o, rays_d, t, dfeat, ctx.geom, g, chunks, done)
+            return ops.hash_bwd_stream_tiles(n_pts)
+
+        if tab.wanted:
+            # the MLP gradient is complete (and published) behind the first level chunk, or travels in the streamed exchange
+            tab.scatter_table(lambda g, l0, l1: ops.hash_encode_bwd_rays(rays_o, rays_d, t, dfeat, ctx.geom, g, l0, l1),
+                              n_pts, stream, after_first=join_mlp, mlp=mlp, mlp_stream=side if defer else None)
         else:
-            g = torch.zeros((L, T, F), device=dout.device, dtype=torch.float32)
-        ops.hash_encode_bwd_rays(rays_o, rays_d, t, dfeat, ctx.geom, g, 0, L)
-        join_mlp()
-        return (None, None, None, ddirs, None, None) + tuple(g[i] for i in range(L)) + gm
+            join_mlp()
+        return (None, None, None, ddirs, None, None) + tab.grads() + mlp.grads()
 
 
 class _FieldCompactFn(torch.autograd.Function):
@@ -232,54 +172,24 @@ class _FieldCompactFn(torch.autograd.Function):
         out, _ = ops.mlp_fwd_tc(feat16, dirs, 1, flat, dims, operand=operand, image_ready=True, n_dev=count, dir_rows=ray_c)
         ctx.enc, ctx.mlp, ctx.geom, ctx.dims, ctx.operand = enc, mlp, geom, dims, operand
         ctx.save_for_backward(pts_c, ray_c, count, dirs, feat16, out)
-        ctx.want_tab = any(ctx.needs_input_grad[9:9 + enc.L])
-        ctx.want_mlp = any(ctx.needs_input_grad[9 + enc.L:])
-        ctx.g = None
-        if ctx.want_tab:
-            if enc._dp is not None:
-                enc._dp.note_forward(enc)
-            else:
-                ctx.g = enc._zeroed_grad_async()
-        if ctx.want_mlp and mlp._dp is not None:
-            mlp._dp.note_forward(mlp)
+        ctx.tab_grad = ParamGrad(enc, any(ctx.needs_input_grad[9:9 + enc.L]))
+        ctx.mlp_grad = ParamGrad(mlp, any(ctx.needs_input_grad[9 + enc.L:]))
         ctx.mark_non_differentiable(rowmap, count)
         return out, rowmap, count
 
     @staticmethod
     def backward(ctx, dout, _g_rowmap, _g_count):
         pts_c, ray_c, count, dirs, feat16, out = ctx.saved_tensors
-        enc, mlp = ctx.enc, ctx.mlp
-        L, T, F = enc.L, enc.T, enc.F
-        flat = mlp._flat_params()
-        dpm = mlp._dp if ctx.want_mlp else None
-        if dpm is not None:
-            dflat, last_m = dpm.enter_backward(mlp)
-        else:
-            dflat, last_m = torch.zeros_like(flat), False
-        dfeat, ddirs = ops.mlp_bwd_tc(feat16, dirs, 1, flat, ctx.dims, out.detach(), dout.float().contiguous(), ctx.want_tab,
-                                      ctx.needs_input_grad[3], dflat, operand=ctx.operand, grad_scale=mlp.tc_grad_scale,
-                                      n_dev=count, dir_rows=ray_c)
-        if dpm is not None and last_m:
-            dpm.publish(mlp, dflat)
-        gm = (None,) * len(mlp._ordered()) if (dpm is not None or not ctx.want_mlp) else tuple(mlp._grad_views(dflat))
-        head = (None, None, None, ddirs, None, None, None, None, None)
-        if not ctx.want_tab:
-            return head + (None,) * L + gm
-        dpe = enc._dp
-        if dpe is not None:
-            g, last = dpe.enter_backward(enc)
-            ops.hash_encode_bwd_pts(pts_c, count, dfeat, ctx.geom, g, 0, L)
-            if last:
-                dpe.publish(enc, g)
-            return head + (None,) * L + gm
-        if ctx.g is not None:
-            g, ev = ctx.g
-            ctx.g = None
-            torch.cuda.current_stream().wait_event(ev)
-        else:
-            g = torch.zeros((L, T, F), device=dout.device, dtype=torch.float32)
-        ops.hash_encode_bwd_pts(pts_c, count, dfeat, ctx.geom, g, 0, L)
-        return head + tuple(g[i] for i in range(L)) + gm
+        tab, mlp = ctx.tab_grad, ctx.mlp_grad
+        dflat = mlp.buffer()
+        dfeat, ddirs = ops.mlp_bwd_tc(feat16, dirs, 1, ctx.mlp._flat_params(), ctx.dims, out.detach(), dout.float().contiguous(),
+                                      tab.wanted, ctx.needs_input_grad[3], dflat, operand=ctx.operand,
+                                      grad_scale=ctx.mlp.tc_grad_scale, n_dev=count, dir_rows=ray_c)
+        mlp.complete()
+        if tab.wanted:
+            ops.hash_encode_bwd_pts(pts_c, count, dfeat, ctx.geom, tab.buffer(), 0, ctx.enc.L)
+            tab.complete()                                 # published whole
+        return (None, None, None, ddirs, None, None, None, None, None) + tab.grads() + mlp.grads()
 
 
 # hbr_field_bwd_rays_tc (MLP backward + hash-grid scatter-add in one kernel) on the single-GPU autocast path; the
@@ -309,14 +219,6 @@ def _side_stream(device) -> torch.cuda.Stream:
     if s is None:
         s = _SIDE[idx] = torch.cuda.Stream(device=idx)
     return s
-
-
-def _field_params(enc, mlp):
-    """The parameters a field autograd node depends on.  Under no_grad they are passed detached: the nodes decide from
-    needs_input_grad (which follows requires_grad, not the grad mode) whether to allocate and zero a table gradient buffer
-    in their forward, and no backward would ever read it."""
-    ps = [*[e.weight for e in enc.Embedding_list], *mlp._ordered()]
-    return ps if torch.is_grad_enabled() else [p.detach() for p in ps]
 
 
 # Volume_Renderer.render: colours, depth and opacity maps of the coarse and the fine pass, the eikonal norms (SDF mode)
@@ -496,11 +398,11 @@ class Volume_Renderer:
             if mask_needed and self.compact and S <= 1024 and R * S < 2 ** 31:
                 mu, sig = self._norm_host()
                 out4, rowmap, _ = _FieldCompactFn.apply(rays_o, rays_d, t.float().contiguous(), dir_enc.float().contiguous(),
-                                                        self.bool_grid, mu, sig, enc, mlp, *_field_params(enc, mlp))
+                                                        self.bool_grid, mu, sig, enc, mlp, *node_params(enc, mlp))
                 return self._composite(out4, t, dir_norm, None, R, S, rowmap, maps)
             mask = self.get_mask(ops.ray_points(rays_o, rays_d, t).view(-1, 3)) if mask_needed else None
             out4 = _FieldRaysFn.apply(rays_o, rays_d, t.float().contiguous(), dir_enc.float().contiguous(), enc, mlp,
-                                      *_field_params(enc, mlp))
+                                      *node_params(enc, mlp))
             return self._composite(out4, t, dir_norm, mask, R, S, None, maps)
         pts = ops.ray_points(rays_o, rays_d, t).view(-1, 3)
         mask = self.get_mask(pts) if mask_needed else None
@@ -508,7 +410,7 @@ class Volume_Renderer:
             enc = self.Pos_encode
             if enc._flat_table().device != pts.device:
                 raise RuntimeError(f"encoder tables are on {enc._flat_table().device}, rays on {pts.device}")
-            out4 = _FieldFn.apply(pts, dir_enc, S, enc, mlp, *_field_params(enc, mlp))
+            out4 = _FieldFn.apply(pts, dir_enc, S, enc, mlp, *node_params(enc, mlp))
         else:
             feat = self.Pos_encode(pts)
             out4 = mlp.field(feat, dir_enc, S)
@@ -688,7 +590,7 @@ class Volume_Renderer:
         pts = ops.ray_points(rays_o, rays_d, t).view(-1, 3)
         if self._can_chain(mlp):
             out4 = _FieldRaysFn.apply(rays_o, rays_d, t.float().contiguous(), dir_enc.float().contiguous(), enc, mlp,
-                                      *_field_params(enc, mlp))
+                                      *node_params(enc, mlp))
         else:
             out4 = mlp.field(enc(pts), dir_enc, S, raw=True)
         Cr, w = ops.CompositeSdfPacked.apply(out4, self.var_model.b, R, S, bool(mlp.use_sdf))
